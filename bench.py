@@ -2,6 +2,7 @@
 """Benchmark of the MoCoPCI neighbourhood hot path on B200 (contract: task brief / DESIGN.md section 7).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--no-extras]
+                    [--dump-outputs DIR]
 
 Headline metric (BASELINE.json): KNN queries/s, k=16, 16384 queries x 16384 refs per frame pair.
 A *step* is one pass of ``knn_point(16, frame t, frame t+1)`` over the rank's batch of synthetic
@@ -23,6 +24,12 @@ there is no data-path collective => weak scaling.
   kernels     (extras, N=1) the other rows of SURVEY section 8d with their own rooflines
 
 ``--impl reference`` times only the CPU path (rank 0; other ranks exit 0).
+
+``--dump-outputs DIR`` writes what the timed KNN call returned in its last timed step, so that two
+builds can be compared output for output (the inputs depend on the rank only): a fixed, seeded
+sample of DUMP_ROWS (frame pair, query) rows of the int64 indices, as float32, to
+DIR/knn_idx.npy (DIR/knn_idx_rank<r>.npy when several ranks run), and the rows' positions as
+DIR/knn_rows.npy (pair index, query index).
 """
 import argparse
 import ctypes
@@ -48,6 +55,7 @@ PAIRS_PER_GPU = 64  # BASELINE config 5's batch; one knn_point call per step
 EVAL_PAIRS = 64
 FLOP_PER_PAIR = 8.0  # SURVEY 8d: 3 sub, 3 mul, 2 add (equivalently the expanded form)
 T_INTERP = [0.4167, 0.5, 0.5833]  # train.py:49-55 with the defaults
+DUMP_ROWS = 65536  # of the 64 x 16384 query rows a step returns: 4 MiB of indices as float32
 
 
 def load_peaks():
@@ -500,6 +508,19 @@ def eval64_leg(net, dist, rank, world):
             "reduce": "one all_reduce(SUM) of a 9-element FP64 vector over NCCL" if dist is not None else "single rank"}
 
 
+def dump_outputs(out_dir, idx, name):
+    """A seeded sample of DUMP_ROWS rows of ``idx`` [pairs, queries, k] (the same rows every run)."""
+    import numpy as np
+    pairs, queries, _ = idx.shape
+    rows = torch.randperm(pairs * queries, generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort()[0]
+    sample = idx.reshape(pairs * queries, -1)[rows.cuda()].float().cpu().numpy()  # indices < 2^24: exact
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"{name}.npy"), sample)
+    if int(os.environ.get("RANK", "0")) == 0:  # the same rows on every rank
+        np.save(os.path.join(out_dir, "knn_rows.npy"),
+                np.stack([(rows // queries).numpy(), (rows % queries).numpy()], 1).astype(np.float64))
+
+
 def run_ours(args):
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -560,10 +581,13 @@ def run_ours(args):
     if rank == 0:
         sampler.start()
     t_warm = time.time()
+    last = None
     while True:  # W warm-up steps, and at least 0.3 s of load so that nvidia-smi is sampling
         for _ in range(max(args.warmup, 3)):
             flush()
-            step()
+            # kept like the timed loop keeps it, so that the allocator already holds the two
+            # output blocks the timed steps alternate between
+            last = step()
         torch.cuda.synchronize()
         if time.time() - t_warm > 0.3:
             break
@@ -575,7 +599,7 @@ def run_ours(args):
         flush()
         e0, e1 = ev_pair()
         e0.record()
-        step()
+        last = step()
         e1.record()
         evs.append((e0, e1))
     barrier()
@@ -585,6 +609,9 @@ def run_ours(args):
     kern_n = int(_lib.lib.b200pci_debug_get(4))
     _lib.check(_lib.lib.b200pci_debug_set(3, 0))
     clocks = sampler.stop(t_region0, t_region1) if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last, "knn_idx" if world == 1 else f"knn_idx_rank{rank}")
+    del last
     total_ms = torch.tensor([sum(step_ms)], dtype=torch.float64, device="cuda")
     if dist is not None:
         dist.all_reduce(total_ms, op=dist.ReduceOp.MAX)
@@ -726,9 +753,12 @@ def main():
     ap.add_argument("--no-eval", action="store_true", help="skip the config-5 eval leg")
     ap.add_argument("--no-parity", action="store_true", help="skip the pre-timing oracle check")
     ap.add_argument("--model-steps", type=int, default=5)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed sample of the last timed step's KNN indices to DIR/*.npy")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the GPU path's outputs; it does not apply to --impl reference")
     if args.impl == "reference":
-        args.steps = min(args.steps, 20)
         return run_reference(args)
     return run_ours(args)
 

@@ -1,4 +1,5 @@
-"""TEST INFRASTRUCTURE ONLY -- torch restatement of the reference's pure-torch CPU KNN/Chamfer path.
+"""TEST INFRASTRUCTURE ONLY -- torch restatement of the reference's pure-torch CPU KNN/Chamfer path
+and of the distance helpers the GPU parity tests run on CUDA tensors.
 
 This is what ``bench.py --impl reference`` and the ``cpu_baseline`` leg time on the GPU box's
 host cores (the reference's Python cannot travel there): the same torch ops, in the same order,
@@ -32,3 +33,17 @@ def chamfer(pc1, pc2):
     y = pc2.permute(0, 2, 1)
     d = square_distance(x, y)
     return (d.min(dim=2)[0].mean(dim=1) + d.min(dim=1)[0].mean(dim=1)).mean()
+
+
+def square_distance_sqdiff(src, dst):
+    # models/pointT_layer2.py:20: sum of squared coordinate differences; CUDA torch adds
+    # (dx^2 + dz^2) + dy^2, CPU torch (dx^2 + dy^2) + dz^2
+    return torch.sum((src[:, :, None] - dst[:, None]) ** 2, dim=-1)
+
+
+def cosine_distance(src, dst):
+    # models/pointconv_util.py:111-127: 1 - <q/|q|, r/|r|> for q in src [B,S,C], r in dst [B,N,C].
+    # Restated from the definition, not op for op: compare with a tolerance
+    src = src / torch.norm(src, dim=-1, keepdim=True)
+    dst = dst / torch.norm(dst, dim=-1, keepdim=True)
+    return 1 - torch.matmul(src, dst.permute(0, 2, 1))

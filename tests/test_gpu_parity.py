@@ -4,7 +4,11 @@ reference-facing Python layer (which goes through the C ABI), against
   * the committed golden fixtures generated from the reference's own torch code, and
   * the reference's own CUDA kernels compiled unmodified into oracle/_ref (bitwise).
 Bar: bit-exact for indices / gathers / distances in the reference arithmetic; 1e-5 relative for
-Chamfer / EMD values (tolerance written at each assert).
+Chamfer / EMD values (tolerance written at each assert). The reference's torch distance helpers
+are restated in oracle/torch_port.py and run on the same CUDA tensors. Where a test compared with
+the reference's compiled kernels, which need a MoCoPCI checkout, it compares with a stored snapshot
+of kernel outputs instead (tests/kernel_snapshot.py), next to the oracle where the oracle covers
+the operator.
 """
 import glob
 import os
@@ -14,6 +18,9 @@ import types
 import numpy as np
 import pytest
 import torch
+
+from oracle import torch_port
+from tests import kernel_snapshot as snapshot
 
 pytestmark = pytest.mark.gpu
 
@@ -44,7 +51,8 @@ class _OwnEmd:
 def ops(request):
     """The operators under test, reached the way a user reaches them:
     * reference_wrappers: the REFERENCE's own pointnet2/pointnet2_utils.py, models/EMD/emd.py and
-      models/utils.py (imported unmodified from the checkout) on top of mocopci_b200.install();
+      models/utils.py (imported unmodified from a checkout when one is available, else their calls
+      restated in tests/refwrappers.py) on top of mocopci_b200.install();
     * own_api: mocopci_b200.ops."""
     if not torch.cuda.is_available():
         pytest.skip("no CUDA device")
@@ -58,14 +66,21 @@ def ops(request):
     o.chamfer, o.emd_cuda, o.pcu, o.p2c, o.synth, o.own = (chamfer, emd_cuda, pointconv_util,
                                                            pointnet2_cuda, synth, own)
     if request.param == "reference_wrappers":
-        root = request.getfixturevalue("ref_root")
-        mocopci_b200.install(reference_root=root)
         import importlib
-        o.p2u = importlib.import_module("pointnet2.pointnet2_utils")
-        assert o.p2u.pointnet2 is pointnet2_cuda          # the reference file runs on our module
-        emd_mod = importlib.import_module("models.EMD.emd")
-        utils = importlib.import_module("models.utils")
-        o.emd = types.SimpleNamespace(earth_mover_distance=emd_mod.earth_mover_distance, EMD=utils.EMD)
+        from baseline import fetch_ref
+        root = fetch_ref.root()
+        mocopci_b200.install(reference_root=root)
+        if root is not None:
+            o.p2u = importlib.import_module("pointnet2.pointnet2_utils")
+            emd_mod = importlib.import_module("models.EMD.emd")
+            utils = importlib.import_module("models.utils")
+            o.emd = types.SimpleNamespace(earth_mover_distance=emd_mod.earth_mover_distance, EMD=utils.EMD)
+        else:
+            from tests import refwrappers
+            o.p2u = refwrappers
+            o.emd = types.SimpleNamespace(earth_mover_distance=refwrappers.earth_mover_distance,
+                                          EMD=refwrappers.EMD)
+        assert o.p2u.pointnet2 is pointnet2_cuda          # the reference's wrappers run on our module
     else:
         o.p2u, o.emd = _OwnP2U(own), _OwnEmd(own)
     return o
@@ -77,6 +92,18 @@ def dev(a):
 
 def bits(a):
     return np.ascontiguousarray(a, dtype=np.float32).view(np.int32)
+
+
+def installed_knn_point():
+    """``knn_point`` as mocopci_b200.install() binds it in the reference's modules; the inputs of the
+    tests that use it are all covered by the kernel, so the reference's own function is never run.
+    install() only re-binds functions of imported reference modules, so without a checkout the
+    binding is made directly with the helper it uses (shim._replacement)."""
+    from mocopci_b200 import shim
+
+    def reference_knn_point(*args):
+        raise AssertionError("the installed knn_point fell back to the reference's torch code")
+    return shim._replacement("knn_point", reference_knn_point)
 
 
 # ------------------------------------------------------------------------------------------
@@ -406,18 +433,13 @@ def test_knn_sqdiff_golden_reference(ops, name):
 @pytest.mark.parametrize("layout", ["contiguous", "permuted", "mixed"])
 @pytest.mark.parametrize("B,S,N,k", [(1, 16384, 16384, 16), (1, 16384, 16384, 32), (2, 4096, 16384, 3),
                                       (1, 2048, 2048, 16), (3, 700, 1000, 8)])
-def test_knn_bitwise_vs_reference_on_the_same_gpu(ops, ref_root, B, S, N, k, layout):
-    """The reference's own square_distance + topk executed by CUDA torch on this GPU
-    (models/pointconv_util.py:67-88,129-140 imported from the checkout, helpers un-patched): our
-    default ("cuda") arithmetic reproduces its matrix entries BITWISE at the selected indices and
-    selects the same k-distance multiset for every query; index sets equal wherever it has no tie."""
-    if ops.api != "own_api":
-        pytest.skip("same kernels; run once")
-    import importlib
-    import mocopci_b200
-    from mocopci_b200 import shim
-    mocopci_b200.install(reference_root=ref_root)
-    ref = importlib.import_module("models.pointconv_util")
+def test_knn_bitwise_vs_reference_on_the_same_gpu(ops, B, S, N, k, layout):
+    """The reference's square_distance + topk (models/pointconv_util.py:67-88,129-140, restated op
+    for op in oracle/torch_port.py) executed by CUDA torch on this GPU: our default ("cuda")
+    arithmetic reproduces its matrix entries BITWISE at the selected indices and selects the same
+    k-distance multiset for every query; index sets equal wherever it has no tie. The
+    reference_wrappers variant calls knn_point as install() binds it in the reference's modules,
+    which returns the indices only."""
     a, b = ops.synth.frame_pairs(50 + k, B, max(S, N))
     xyz, new = a[:, :N].contiguous().cuda(), b[:, :S].contiguous().cuda()
     # the model mostly passes permuted views of [B,3,N] tensors (mocopci.py:1327); CUDA torch's
@@ -426,29 +448,29 @@ def test_knn_bitwise_vs_reference_on_the_same_gpu(ops, ref_root, B, S, N, k, lay
         new = new.permute(0, 2, 1).contiguous().permute(0, 2, 1)
     if layout == "permuted":
         xyz = xyz.permute(0, 2, 1).contiguous().permute(0, 2, 1)
-    D = getattr(ref.square_distance, shim._MARK, ref.square_distance)(new, xyz)
-    idx, dist = ops.pcu.knn_point_with_dist(k, xyz, new)
-    assert torch.equal(torch.gather(D, 2, idx).view(torch.int32), dist.view(torch.int32))
+    D = torch_port.square_distance(new, xyz)
+    if ops.api != "own_api":
+        idx = installed_knn_point()(k, xyz, new)
+        dist = torch.gather(D, 2, idx)
+    else:
+        idx, dist = ops.pcu.knn_point_with_dist(k, xyz, new)
+        assert torch.equal(torch.gather(D, 2, idx).view(torch.int32), dist.view(torch.int32))
     vals = torch.topk(D, k + 1, dim=-1, largest=False, sorted=True)[0]
     assert torch.equal(vals[..., :k].view(torch.int32), dist.view(torch.int32))
-    ref_idx = getattr(ref.knn_point, shim._MARK)(k, xyz, new)
+    ref_idx = torch_port.knn_point(k, xyz, new)
     no_tie = vals[..., k - 1] != vals[..., k]
     assert bool((idx.sort(-1)[0] == ref_idx.sort(-1)[0]).all(-1)[no_tie].all())
 
 
 @pytest.mark.parametrize("permuted", [False, True])
-def test_knn_sqdiff_bitwise_vs_reference_on_the_same_gpu(ops, ref_root, permuted):
-    """f3 on the GPU: models/pointT_layer2.py:20,62-63 executed by CUDA torch (its 3-element sum adds
-    (dx^2 + dz^2) + dy^2, unlike the CPU): same ascending distances bit for bit."""
-    import importlib
-    import mocopci_b200
-    from mocopci_b200 import shim
-    mocopci_b200.install(reference_root=ref_root)
-    pt = importlib.import_module("models.pointT_layer2")
+def test_knn_sqdiff_bitwise_vs_reference_on_the_same_gpu(ops, permuted):
+    """f3 on the GPU: models/pointT_layer2.py:20,62-63 (restated in oracle/torch_port.py) executed by
+    CUDA torch (its 3-element sum adds (dx^2 + dz^2) + dy^2, unlike the CPU): same ascending
+    distances bit for bit."""
     xyz = ops.synth.lidar_frame(99, 2048)[None].cuda()
     if permuted:
         xyz = xyz.permute(0, 2, 1).contiguous().permute(0, 2, 1)
-    D = getattr(pt.square_distance, shim._MARK, pt.square_distance)(xyz, xyz)
+    D = torch_port.square_distance_sqdiff(xyz, xyz)
     ref_sorted = D.sort(-1)[0][:, :, :17]
     idx = ops.pcu.knn_point_sqdiff(16, xyz, xyz)
     assert torch.equal(torch.gather(D, 2, idx).view(torch.int32), ref_sorted[..., :16].view(torch.int32))
@@ -475,10 +497,14 @@ def test_knn_direct_forms_vs_oracle(ops, orc, form, B, S, N, k):
 @pytest.mark.parametrize("k", [16, 32])
 def test_knn_full_benchmark_pair_vs_oracle(ops, orc, k):
     """One full 16384 x 16384 frame pair of the BENCHMARKED workload (bench.py: synth.frame_pairs(0, .))
-    against the OpenMP C oracle: every index and every distance bit."""
-    if ops.api != "own_api":
-        pytest.skip("same kernels; run once")
+    against the OpenMP C oracle: every index and every distance bit. The reference_wrappers variant
+    calls knn_point as install() binds it in the reference's modules: every index, in the
+    reference's CUDA torch arithmetic (oracle form 5)."""
     a, b = ops.synth.frame_pairs(0, 1)
+    if ops.api != "own_api":
+        idx = installed_knn_point()(k, dev(a), dev(b))
+        np.testing.assert_array_equal(idx.cpu().numpy(), orc.knn_form(5, k, a.numpy(), b.numpy())[0])
+        return
     check_knn_against_oracle(ops, orc, a.numpy(), b.numpy(), k)
 
 
@@ -534,7 +560,7 @@ COS_GAP = 8e-6    # order (and the tensor core truncates when aligning addends: 
 
 
 def check_cosine(idx, dist, ref_D, k):
-    """ref_D: the REFERENCE's cosine_distance matrix [B,S,N] (torch). (i) our k distances equal the
+    """ref_D: the reference's cosine_distance matrix [B,S,N] (torch). (i) our k distances equal the
     reference's k smallest to COS_ATOL, and are what the reference has at our indices; (ii) same
     index set wherever the reference's k-th and (k+1)-th distances are more than COS_GAP apart."""
     kk = min(k + 1, ref_D.shape[-1])
@@ -570,13 +596,10 @@ def test_knn_point_cosine_golden_reference(ops, path):
                                                  (1, 256, 256, 256, 16, True), (2, 300, 1000, 64, 16, False),
                                                  (1, 129, 4096, 32, 32, False), (3, 77, 257, 16, 5, True),
                                                  (1, 1, 16, 512, 16, False), (2, 1000, 130, 48, 32, True)])
-def test_knn_point_cosine_vs_reference_function(ops, orc, ref_root, B, S, N, C, k, permuted):
-    """Against the REFERENCE's own cosine_distance + topk executed on the same GPU
-    (models/pointconv_util.py:111-127,142-153 imported from the checkout) and against the oracle."""
-    import importlib
-    import mocopci_b200
-    mocopci_b200.install(reference_root=ref_root)
-    ref = importlib.import_module("models.pointconv_util")
+def test_knn_point_cosine_vs_reference_function(ops, orc, B, S, N, C, k, permuted):
+    """Against the reference's cosine_distance + topk (models/pointconv_util.py:111-127,142-153,
+    restated in oracle/torch_port.py) executed by CUDA torch on the same GPU, every row, and
+    against the oracle; with a checkout, the installed helper too."""
     g = torch.Generator().manual_seed(B * 1000 + S + N + C)
     xyz = torch.randn(B, C, N, generator=g) if permuted else torch.randn(B, N, C, generator=g)
     new = torch.randn(B, C, S, generator=g) if permuted else torch.randn(B, S, C, generator=g)
@@ -584,22 +607,25 @@ def test_knn_point_cosine_vs_reference_function(ops, orc, ref_root, B, S, N, C, 
     nd = new.cuda().permute(0, 2, 1) if permuted else new.cuda()
     idx, dist = ops.pcu.knn_point_cosine_with_dist(k, xd, nd)
     assert idx.dtype == torch.int64 and tuple(idx.shape) == (B, S, k)
-    frac = check_cosine(idx, dist, ref.cosine_distance(nd, xd), k)
+    frac = check_cosine(idx, dist, torch_port.cosine_distance(nd, xd), k)
     assert frac > 0.8
-    # the installed replacement routes through the same kernel and returns the same indices
-    assert hasattr(ref.knn_point_cosine, "__b200pci_original__")
-    assert torch.equal(ref.knn_point_cosine(k, xd, nd), idx)
     oi, od = orc.knn_cosine(k, xd.contiguous().cpu().numpy(), nd.contiguous().cpu().numpy())
     np.testing.assert_allclose(dist.cpu().numpy(), od, rtol=0, atol=COS_ATOL)
+    from baseline import fetch_ref
+    if fetch_ref.root() is not None:
+        # the installed replacement routes through the same kernel and returns the same indices
+        import importlib
+        import mocopci_b200
+        mocopci_b200.install(reference_root=fetch_ref.root())
+        ref = importlib.import_module("models.pointconv_util")
+        assert hasattr(ref.knn_point_cosine, "__b200pci_original__")
+        assert torch.equal(ref.knn_point_cosine(k, xd, nd), idx)
 
 
-def test_knn_point_cosine_duplicates_and_unsupported(ops, ref_root):
+def test_knn_point_cosine_duplicates_and_unsupported(ops):
     """Duplicated feature rows (duplicated points) are exact ties: the lowest index wins. Shapes the
-    kernel does not cover fall back to the reference's own torch code through the installed helper."""
-    import importlib
-    import mocopci_b200
-    mocopci_b200.install(reference_root=ref_root)
-    ref = importlib.import_module("models.pointconv_util")
+    kernel does not cover raise; with a checkout, they fall back to the reference's own torch code
+    through the installed helper."""
     g = torch.Generator().manual_seed(5)
     base = torch.randn(1, 300, 64, generator=g)
     xyz = torch.cat([base, base], 1).cuda()          # ref j and j + 300 are identical
@@ -609,10 +635,16 @@ def test_knn_point_cosine_duplicates_and_unsupported(ops, ref_root):
     assert float(dist[0, :, :2].abs().max()) <= COS_ATOL
     odd = torch.randn(1, 100, 50, generator=g).cuda()                            # C % 16 != 0
     assert not ops.pcu.cosine_supported(8, odd, odd)
-    out = ref.knn_point_cosine(8, odd, odd)                                      # the reference's own code
-    assert tuple(out.shape) == (1, 100, 8)
     with pytest.raises(RuntimeError):
         ops.pcu.knn_point_cosine(8, odd, odd)
+    from baseline import fetch_ref
+    if fetch_ref.root() is not None:
+        import importlib
+        import mocopci_b200
+        mocopci_b200.install(reference_root=fetch_ref.root())
+        ref = importlib.import_module("models.pointconv_util")
+        out = ref.knn_point_cosine(8, odd, odd)                                  # the reference's own code
+        assert tuple(out.shape) == (1, 100, 8)
 
 
 def test_knn_k_gt_n_raises(ops):
@@ -671,16 +703,20 @@ def test_three_nn(ops, orc, B, n, m, request):
     np.testing.assert_array_equal(bits(dist.cpu().numpy()), bits(np.sqrt(od2)))
 
 
-def test_three_nn_vs_reference_kernel(ops, refgpu):
+def test_three_nn_vs_reference_kernel(ops, orc):
+    """The pybind-style entry point on a LiDAR frame: the oracle's squared distances and indices bit
+    for bit, and the kernel snapshot."""
     a, _ = ops.synth.frame_pair(1, 4096)
     known = a[:1024][None].cuda().contiguous()
     unknown = a[None].cuda().contiguous()
     d2 = torch.empty((1, 4096, 3), device="cuda")
     idx = torch.empty((1, 4096, 3), dtype=torch.int32, device="cuda")
     ops.p2c.three_nn_wrapper(1, 4096, 1024, unknown, known, d2, idx)
-    rd2, ridx = refgpu.three_nn(unknown, known)
-    assert torch.equal(idx, ridx)
-    assert torch.equal(d2.view(torch.int32), rd2.view(torch.int32))
+    od2, oi = orc.three_nn(unknown.cpu().numpy(), known.cpu().numpy())
+    np.testing.assert_array_equal(idx.cpu().numpy(), oi)
+    np.testing.assert_array_equal(bits(d2.cpu().numpy()), bits(od2))
+    snapshot.check("three_nn/idx", idx)
+    snapshot.check("three_nn/d2", d2)
 
 
 @pytest.mark.parametrize("B,n,m", [(2, 256, 64), (1, 4096, 1024), (1, 16384, 4096), (1, 50, 3)])
@@ -705,7 +741,7 @@ def test_three_nn_weights_fused(ops, orc, B, n, m):
 
 @pytest.mark.parametrize("B,C,m,n", [(2, 128, 64, 256), (1, 5, 33, 1000), (2, 19, 1024, 4096),
                                      (1, 128, 4096, 16384), (2, 64, 1000, 5000)])
-def test_three_interpolate_fwd_bwd(ops, orc, refgpu, B, C, m, n):
+def test_three_interpolate_fwd_bwd(ops, orc, B, C, m, n):
     g = torch.Generator().manual_seed(C)
     feat = torch.randn(B, C, m, generator=g)
     idx = torch.randint(0, m, (B, n, 3), generator=g, dtype=torch.int32)
@@ -715,8 +751,7 @@ def test_three_interpolate_fwd_bwd(ops, orc, refgpu, B, C, m, n):
     out = ops.p2u.three_interpolate(fd, idx.cuda(), w.cuda())
     ref = orc.three_interpolate(feat.numpy(), idx.numpy(), w.numpy())
     np.testing.assert_array_equal(bits(out.detach().cpu().numpy()), bits(ref))      # bitwise
-    assert torch.equal(out.detach().view(torch.int32),
-                       refgpu.three_interpolate(feat.cuda(), idx.cuda(), w.cuda()).view(torch.int32))
+    snapshot.check(f"three_interpolate/{B}-{C}-{m}-{n}", out)
     go = torch.randn(B, C, n, generator=g)
     out.backward(go.cuda())
     gref = orc.three_interpolate_grad(go.numpy(), idx.numpy(), w.numpy(), m)
@@ -728,14 +763,14 @@ def test_three_interpolate_fwd_bwd(ops, orc, refgpu, B, C, m, n):
 # gather / group (F2, G1, K3, K4)
 # ------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("B,C,N,M", [(2, 3, 1000, 256), (1, 64, 4096, 1023), (3, 17, 50, 7)])
-def test_gather_fwd_bwd(ops, orc, refgpu, B, C, N, M):
+def test_gather_fwd_bwd(ops, orc, B, C, N, M):
     g = torch.Generator().manual_seed(N)
     feat = torch.randn(B, C, N, generator=g)
     idx = torch.randint(0, N, (B, M), generator=g, dtype=torch.int32)
     fd = feat.cuda().requires_grad_(True)
     out = ops.p2u.gather_operation(fd, idx.cuda())
     np.testing.assert_array_equal(out.detach().cpu().numpy(), orc.gather(feat.numpy(), idx.numpy()))
-    assert torch.equal(out.detach(), refgpu.gather(feat.cuda(), idx.cuda()))
+    snapshot.check(f"gather/{B}-{C}-{N}-{M}", out)
     go = torch.randn(B, C, M, generator=g)
     out.backward(go.cuda())
     np.testing.assert_allclose(fd.grad.cpu().numpy(), orc.gather_grad(go.numpy(), idx.numpy(), N),
@@ -744,14 +779,14 @@ def test_gather_fwd_bwd(ops, orc, refgpu, B, C, N, M):
 
 @pytest.mark.parametrize("B,C,N,np_,ns", [(2, 3, 1000, 128, 32), (1, 35, 2048, 300, 16),
                                            (2, 7, 64, 33, 3), (1, 128, 4096, 1024, 32)])
-def test_group_fwd_bwd(ops, orc, refgpu, B, C, N, np_, ns):
+def test_group_fwd_bwd(ops, orc, B, C, N, np_, ns):
     g = torch.Generator().manual_seed(np_)
     feat = torch.randn(B, C, N, generator=g)
     idx = torch.randint(0, N, (B, np_, ns), generator=g, dtype=torch.int32)
     fd = feat.cuda().requires_grad_(True)
     out = ops.p2u.grouping_operation(fd, idx.cuda())
     np.testing.assert_array_equal(out.detach().cpu().numpy(), orc.group(feat.numpy(), idx.numpy()))
-    assert torch.equal(out.detach(), refgpu.group(feat.cuda(), idx.cuda()))
+    snapshot.check(f"group/{B}-{C}-{N}-{np_}-{ns}", out)
     go = torch.randn(B, C, np_, ns, generator=g)
     out.backward(go.cuda())
     np.testing.assert_allclose(fd.grad.cpu().numpy(), orc.group_grad(go.numpy(), idx.numpy(), N),
@@ -805,14 +840,13 @@ def test_index_points_group_fused_fwd_bwd(ops, B, N, S, K, C, permuted):
                                                  (1, 64, 64, 64, 5, False), (1, 100, 33, 5, 6, False),
                                                  (1, 256, 64, 4, 700, False), (1, 128, 16, 4, 3000, False),
                                                  (1, 512, 512, 16, 128, True)])
-def test_group_query_fused(ops, ref_root, B, N, S, K, D, permuted):
+def test_group_query_fused(ops, orc, B, N, S, K, D, permuted):
     """f1: group / group_query (models/pointconv_util.py:194-241) as ONE gather-subtract-concatenate
     kernel after the neighbour search, bitwise against the composition the reference writes
     (gather xyz - centre | gather points) on the same indices; the autograd path gives the same values;
-    and the reference's own group_query (imported, unpatched) agrees as neighbour SETS."""
-    import importlib
-    import mocopci_b200
-    from mocopci_b200 import shim
+    and the neighbours are those of the reference's knn_point in its CUDA torch arithmetic (the
+    oracle's form 5); with a checkout, the reference's own group_query (imported, unpatched)
+    agrees as neighbour SETS."""
     g = torch.Generator().manual_seed(N + S + D)
     s_xyz = (torch.rand(B, N, 3, generator=g) * 10).cuda()
     xyz = s_xyz if S == N else (torch.rand(B, S, 3, generator=g) * 10).cuda()
@@ -835,8 +869,15 @@ def test_group_query_fused(ops, ref_root, B, N, S, K, D, permuted):
         assert torch.equal(np2.detach(), new_points) and torch.equal(rel2, rel)
         np2.sum().backward()
         assert pg.grad is not None and float(pg.grad.abs().sum()) > 0
+    np.testing.assert_array_equal(idx.cpu().numpy(), orc.knn_form(5, K, s_xyz.cpu().numpy(), xyz.cpu().numpy())[0])
+    from baseline import fetch_ref
+    if fetch_ref.root() is None:
+        return
     # the reference's own function (torch KNN, unsorted neighbours): same sets per query
-    mocopci_b200.install(reference_root=ref_root)
+    import importlib
+    import mocopci_b200
+    from mocopci_b200 import shim
+    mocopci_b200.install(reference_root=fetch_ref.root())
     ref = importlib.import_module("models.pointconv_util")
     orig = getattr(ref.group_query, shim._MARK)
     saved = {n: getattr(ref, n) for n in ("knn_point", "index_points_group")}
@@ -870,13 +911,12 @@ def test_fps_vs_oracle(ops, orc, B, N, M):
     np.testing.assert_array_equal(idx.cpu().numpy(), oi)
 
 
-def test_fps_ties_vs_reference_kernel(ops, orc, refgpu):
+def test_fps_ties_vs_reference_kernel(ops, orc):
     # integer grid with duplicates: many exactly equal distances -> exercises the tie order
     for N, M in ((1200, 200), (512, 128), (3000, 256)):
         xyz = ops.synth.tie_stress_cloud(N, 2, N, grid=3).cuda()
         idx = ops.p2u.furthest_point_sample(xyz, M)
-        ridx, rtemp = refgpu.fps(xyz, M)
-        assert torch.equal(idx, ridx), f"N={N}"
+        snapshot.check(f"fps_ties/{N}-{M}", idx)
         np.testing.assert_array_equal(idx.cpu().numpy(), orc.fps(xyz.cpu().numpy(), M)[0])
 
 
@@ -895,15 +935,18 @@ def test_fps_single_cta_and_cluster_kernels_agree(ops, orc):
             np.testing.assert_array_equal(a.cpu().numpy(), orc.fps(xyz.cpu().numpy(), M)[0])
 
 
-def test_fps_full_size_vs_reference_kernel(ops, refgpu):
+def test_fps_full_size_vs_reference_kernel(ops, orc):
+    """16384 -> 4096 on two LiDAR frames: the oracle's indices, and indices and the distance buffer
+    bit for bit against the kernel snapshot."""
     a, _ = ops.synth.frame_pairs(0, 2)
+    oi = orc.fps(a.numpy(), 4096)[0]
     a = a.cuda()
     temp = torch.full((2, 16384), 1e10, device="cuda")
     idx = torch.empty((2, 4096), dtype=torch.int32, device="cuda")
     ops.p2c.furthest_point_sampling_wrapper(2, 16384, 4096, a, temp, idx)
-    ridx, rtemp = refgpu.fps(a, 4096)
-    assert torch.equal(idx, ridx)
-    assert torch.equal(temp.view(torch.int32), rtemp.view(torch.int32))
+    np.testing.assert_array_equal(idx.cpu().numpy(), oi)
+    snapshot.check("fps_full/idx", idx)
+    snapshot.check("fps_full/temp", temp)
 
 
 # ------------------------------------------------------------------------------------------
@@ -937,7 +980,7 @@ def test_ball_query_dense_and_forced_redo(ops, orc):
 
 
 @pytest.mark.parametrize("r,ns,shift", [(3.0, 128, 0.0), (1.5, 128, 0.0), (0.4, 96, 500.0), (6.0, 200, 0.0)])
-def test_ball_query_large_nsample_split_overflow(ops, orc, refgpu, r, ns, shift):
+def test_ball_query_large_nsample_split_overflow(ops, orc, r, ns, shift):
     """nsample > the 96-entry pending lists with the refs split over several CTAs (16384 refs, few
     queries): a split whose list overflowed must send the query to the exact redo instead of
     letting later splits fill the slots with higher indices. `shift` moves the cloud far from the
@@ -947,30 +990,36 @@ def test_ball_query_large_nsample_split_overflow(ops, orc, refgpu, r, ns, shift)
     new = a[:, ::40].contiguous()                      # 410 queries: B*M small -> nsplit > 1
     got = ops.p2u.ball_query(r, ns, a.cuda(), new.cuda())
     np.testing.assert_array_equal(got.cpu().numpy(), orc.ball_query(r, ns, a.numpy(), new.numpy()))
-    assert torch.equal(got, refgpu.ball_query(r, ns, a.cuda(), new.cuda()))
+    snapshot.check(f"ball_query_split/{r}-{ns}-{shift}", got)
 
 
-def test_ball_query_lidar_vs_reference_kernel(ops, refgpu):
+def test_ball_query_lidar_vs_reference_kernel(ops, orc):
     a, _ = ops.synth.frame_pairs(2, 2, 8192)
     a = a.cuda()
     centres = ops.pcu.index_points_gather(a, ops.p2u.furthest_point_sample(a, 1024))
     idx = ops.p2u.ball_query(0.5, 32, a, centres)
-    assert torch.equal(idx, refgpu.ball_query(0.5, 32, a, centres))
+    np.testing.assert_array_equal(idx.cpu().numpy(), orc.ball_query(0.5, 32, a.cpu().numpy(), centres.cpu().numpy()))
+    snapshot.check("ball_query_lidar", idx)
     # no-hit rows stay all zero (pointnet2_utils.py:218)
     far = centres + 1000.0
     assert int(ops.p2u.ball_query(0.5, 32, a, far).abs().sum()) == 0
 
 
-def test_query_and_group(ops, refgpu):
+def test_query_and_group(ops, orc):
     a, _ = ops.synth.frame_pairs(4, 1, 4096)
     a = a.cuda()
-    feats = torch.randn(1, 16, 4096, device="cuda")
+    feats = torch.randn(1, 16, 4096, generator=torch.Generator().manual_seed(4)).cuda()
     centres = ops.pcu.index_points_gather(a, ops.p2u.furthest_point_sample(a, 256))
     out = ops.p2u.QueryAndGroup(2.0, 16)(a, centres, feats)
     assert tuple(out.shape) == (1, 19, 256, 16)
-    idx = refgpu.ball_query(2.0, 16, a, centres)
-    gx = refgpu.group(a.transpose(1, 2).contiguous(), idx) - centres.transpose(1, 2).unsqueeze(-1)
-    assert torch.equal(out[:, :3], gx) and torch.equal(out[:, 3:], refgpu.group(feats, idx))
+    # pointnet2_utils.py:250-264 on the oracle: ball_query, group of the cloud minus the centres |
+    # group of the features
+    a_np, c_np = a.cpu().numpy(), centres.cpu().numpy()
+    oidx = orc.ball_query(2.0, 16, a_np, c_np)
+    gx = orc.group(np.ascontiguousarray(a_np.transpose(0, 2, 1)), oidx) - c_np.transpose(0, 2, 1)[..., None]
+    want = np.concatenate([gx, orc.group(feats.cpu().numpy(), oidx)], 1)
+    np.testing.assert_array_equal(bits(out.cpu().numpy()), bits(want))
+    snapshot.check("query_and_group", out)
 
 
 @pytest.mark.parametrize("B,N,M,ns,C,use_xyz", [(2, 4096, 512, 32, 64, True), (1, 1000, 77, 5, 3, True),
@@ -982,9 +1031,8 @@ def test_query_group_fused_equals_reference_composition(ops, B, N, M, ns, C, use
     pointnet2_utils.py:250-264 -- grouping_operation on the transposed cloud, minus the centres,
     grouping_operation on the features, torch.cat -- on the same ball_query indices, for group
     counts that are not multiples of four (scalar tail), without features and without xyz; and the
-    autograd route (inputs that require grad) gives the same values."""
-    if ops.api != "own_api":
-        pytest.skip("own API only: the reference's QueryAndGroup module is tested above")
+    autograd route (inputs that require grad) gives the same values. The reference_wrappers variant
+    takes the composition from the reference's QueryAndGroup module itself."""
     from mocopci_b200 import ops as own
     g = torch.Generator().manual_seed(N + M + C)
     xyz = (torch.rand(B, N, 3, generator=g) * 8).cuda()
@@ -995,6 +1043,10 @@ def test_query_group_fused_equals_reference_composition(ops, B, N, M, ns, C, use
     rel = own.grouping_operation(xyz.transpose(1, 2).contiguous(), idx) - centres.transpose(1, 2).unsqueeze(-1)
     want = rel if feats is None else (torch.cat([rel, own.grouping_operation(feats, idx)], 1) if use_xyz
                                       else own.grouping_operation(feats, idx))
+    if ops.api != "own_api":
+        ref = ops.p2u.QueryAndGroup(1.0, ns, use_xyz=use_xyz)(xyz, centres, feats)
+        assert torch.equal(ref, want)
+        want = ref
     assert got.is_contiguous() and got.shape == want.shape and torch.equal(got, want)
     if feats is not None:
         fg = feats.clone().requires_grad_(True)
@@ -1062,44 +1114,49 @@ def test_emd_known_answer(ops):
 
 
 @pytest.mark.parametrize("B,n,m", [(2, 256, 256), (1, 1000, 500), (2, 300, 1200), (1, 2048, 2048)])
-def test_emd_vs_reference_kernel(ops, refgpu, B, n, m):
+def test_emd_vs_reference_kernel(ops, orc, B, n, m):
+    """approxmatch / matchcost / matchcost_backward against the kernel snapshot (match and grad1 bit
+    for bit), and the cost against the oracle (libm expf there, ex2.approx here: 1e-3 relative)."""
     x1 = (ops.synth.uniform_cloud(n, B, n) * 0.5).cuda()
     x2 = (ops.synth.uniform_cloud(m + 3, B, m) * 0.5).cuda()
+    key = f"emd/{B}-{n}-{m}"
     match = ops.emd_cuda.approxmatch_forward(x1, x2)
-    rmatch = refgpu.emd_approxmatch(x1, x2)
-    assert torch.equal(match.view(torch.int32), rmatch.view(torch.int32))   # bitwise
+    snapshot.check(key + "/match", match)                                   # bitwise
     cost = ops.emd_cuda.matchcost_forward(x1, x2, match)
-    rcost = refgpu.emd_matchcost(x1, x2, rmatch)
-    np.testing.assert_allclose(cost.cpu().numpy(), rcost.cpu().numpy(), rtol=1e-5)  # 1e-5 relative
-    gc = torch.rand(B, device="cuda") + 0.5
+    snapshot.check(key + "/cost", cost, rtol=1e-5)                          # 1e-5 relative
+    x1n, x2n = x1.cpu().numpy(), x2.cpu().numpy()
+    np.testing.assert_allclose(cost.cpu().numpy(), orc.emd_matchcost(x1n, x2n, orc.emd_approxmatch(x1n, x2n)),
+                               rtol=1e-3)
+    gc = (torch.rand(B, generator=torch.Generator().manual_seed(n + m)) + 0.5).cuda()
     g1, g2 = ops.emd_cuda.matchcost_backward(gc, x1, x2, match)
-    r1, r2 = refgpu.emd_matchcost_grad(gc, x1, x2, rmatch)
-    assert torch.equal(g1.view(torch.int32), r1.view(torch.int32))
-    np.testing.assert_allclose(g2.cpu().numpy(), r2.cpu().numpy(), rtol=1e-4, atol=1e-6)
+    snapshot.check(key + "/grad1", g1)
+    snapshot.check(key + "/grad2", g2, rtol=1e-4, atol=1e-6)
 
 
 @pytest.mark.parametrize("B,n,m", [(2, 256, 256), (1, 1000, 500), (2, 300, 1200), (1, 4096, 4096)])
-def test_emd_cost_fused_vs_reference_kernel(ops, refgpu, B, n, m):
-    """Forward-only emd_cost (no match matrix) against the reference's approxmatch + matchcost
-    kernels: 1e-5 relative (north_star's tolerance for EMD values)."""
+def test_emd_cost_fused_vs_reference_kernel(ops, B, n, m):
+    """Forward-only emd_cost (no match matrix) against approxmatch + matchcost, in the kernel
+    snapshot and run now: 1e-5 relative (north_star's tolerance for EMD values)."""
     x1 = (ops.synth.uniform_cloud(n + 1, B, n) * 0.5).cuda()
     x2 = (ops.synth.uniform_cloud(m + 4, B, m) * 0.5).cuda()
     cost = ops.emd_cuda.emd_cost(x1, x2)
-    rcost = refgpu.emd_matchcost(x1, x2, refgpu.emd_approxmatch(x1, x2))
-    np.testing.assert_allclose(cost.cpu().numpy(), rcost.cpu().numpy(), rtol=1e-5)
+    snapshot.check(f"emd_cost/{B}-{n}-{m}", cost, rtol=1e-5)
     mine = ops.emd_cuda.matchcost_forward(x1, x2, ops.emd_cuda.approxmatch_forward(x1, x2))
     np.testing.assert_allclose(cost.cpu().numpy(), mine.cpu().numpy(), rtol=1e-5)
 
 
-def test_emd_metric_vs_reference_kernel(ops, refgpu):
+def test_emd_metric_vs_reference_kernel(ops, orc):
     """E4: EMD(pc1, pc2) = mean(cost) / M (models/utils.py:223-235) on a LiDAR frame pair, through the
-    API under test, against the same formula on the reference kernels' cost: 1e-5 relative."""
+    API under test, against the same formula on the kernel snapshot's cost (1e-5 relative) and on
+    the oracle's (1e-3 relative: libm expf there, ex2.approx here)."""
     a, b = ops.synth.frame_pair(0, 4096)
     pc1, pc2 = a.cuda().T[None].contiguous(), b.cuda().T[None].contiguous()
     v = ops.emd.EMD(pc1, pc2)
-    x1, x2 = a.cuda()[None].contiguous(), b.cuda()[None].contiguous()
-    ref = refgpu.emd_matchcost(x1, x2, refgpu.emd_approxmatch(x1, x2)).mean() / 4096
+    ref = snapshot.get("emd_metric")[0]
     assert abs(float(v) - float(ref)) <= 1e-5 * abs(float(ref))
+    x1, x2 = a[None].numpy(), b[None].numpy()
+    oref = float(orc.emd_matchcost(x1, x2, orc.emd_approxmatch(x1, x2)).mean()) / 4096
+    assert abs(float(v) - oref) <= 1e-3 * abs(oref)
 
 
 def test_emd_vs_oracle_small(ops, orc):

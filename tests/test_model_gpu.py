@@ -82,10 +82,14 @@ def _load_reference_stack(ref_root):
 
 
 @pytest.fixture(scope="module")
-def reference_outputs(ref_root, refgpu):
+def reference_outputs(ref_root):
     """One shadow-mode forward and one plain reference-stack forward (same weights, same input)."""
+    from tests import refgpu
     if not torch.cuda.is_available():
         pytest.skip("no CUDA device")
+    if not refgpu.available():   # a checkout is there: its kernels must be too, or the test would vanish
+        pytest.fail("oracle/_ref/libref_*.so missing next to a MoCoPCI checkout: build them with "
+                    "make -C oracle ref REF=<checkout>")
     rs = _load_reference_stack(ref_root)
     x1, x2 = _frames(NPTS)
     net = _build()
