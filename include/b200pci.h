@@ -219,6 +219,10 @@ int b200pci_group_concat(int B, int N, int S, int K, int D, const float *xyz, in
 /* x [B,N,3], y [B,M,3] (strided like b200pci_knn). Outputs: per-point squared NN distance and   */
 /* NN index in each direction (dist_x [B,N], idx_x int32 [B,N], dist_y [B,M], idx_y [B,M]) and   */
 /* loss[0] = mean_b(mean_i dist_x + mean_j dist_y) accumulated in FP64 then rounded.             */
+/* Both searches are K = 1 in DIST_DIRECT_XYZ, pytorch3d's fma(dz,dz,fma(dy,dy,dx*dx)) with      */
+/* d = point - candidate; among equal distances the lowest index wins. So dist_x / idx_x equal   */
+/* b200pci_knn(K=1, DIST_DIRECT_XYZ) with queries x and refs y bit for bit (knn_points), and     */
+/* dist_y / idx_y the same with x and y exchanged.                                              */
 /* ------------------------------------------------------------------------------------------ */
 size_t b200pci_chamfer_workspace_bytes(int B, int N, int M);
 int b200pci_chamfer_forward(int B, int N, int M,

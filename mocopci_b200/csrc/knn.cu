@@ -1566,10 +1566,12 @@ extern "C" int b200pci_chamfer_forward(int B, int N, int M, const float *x, int6
     const size_t pbytes = align_up((size_t)B * sizeof(double), 256);
     double *partial = reinterpret_cast<double *>(workspace);
     char *ws = reinterpret_cast<char *>(workspace) + pbytes;
-    int rc = knn_impl(B, N, M, 1, B200PCI_DIST_DIRECT, x, x_sb, x_sp, x_sc, y, y_sb, y_sp, y_sc,
+    // pytorch3d's arithmetic, like knn_points: the per-point minima and NN indices are those of
+    // knn_points(x, y, K=1) and knn_points(y, x, K=1) bit for bit
+    int rc = knn_impl(B, N, M, 1, B200PCI_DIST_DIRECT_XYZ, x, x_sb, x_sp, x_sc, y, y_sb, y_sp, y_sc,
                       idx_x, 0, dist_x, ws, workspace_bytes - pbytes, st);
     if (rc) return rc;
-    rc = knn_impl(B, M, N, 1, B200PCI_DIST_DIRECT, y, y_sb, y_sp, y_sc, x, x_sb, x_sp, x_sc, idx_y,
+    rc = knn_impl(B, M, N, 1, B200PCI_DIST_DIRECT_XYZ, y, y_sb, y_sp, y_sc, x, x_sb, x_sp, x_sc, idx_y,
                   0, dist_y, ws, workspace_bytes - pbytes, st);
     if (rc) return rc;
     chamfer_reduce_kernel<<<B, 1024, 0, st>>>(B, N, M, dist_x, dist_y, partial);
