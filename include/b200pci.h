@@ -237,6 +237,53 @@ int b200pci_chamfer_backward(int B, int N, int M, const float *x, const float *y
                              float *grad_x, float *grad_y, void *stream);
 
 /* ------------------------------------------------------------------------------------------ */
+/* D1: deterministic gradients (_det). The scatter-add backwards above add their contributions   */
+/* with float atomics, so the last bits of a gradient vary from run to run. Each _det twin takes */
+/* the same arguments plus device scratch and gives the same sums in ONE fixed order: every      */
+/* destination element is accumulated sequentially in FP32, starting from the value the output  */
+/* holds (callers pre-zero it; Chamfer overwrites), contributions in ascending source position,  */
+/* each product rounded before it is added (no FMA). Every such sum is one of the orders the     */
+/* atomic kernels can produce. Bit for bit reproducible across runs, streams and GPUs of one     */
+/* architecture. Entries of idx outside [0, N) contribute nothing.                               */
+/* Scratch: an inverse index (CSR) of idx per cloud, built on the stream from integer counts;    */
+/* no allocation, no host synchronisation (stream-ordered, graph capturable).                    */
+/* Returns EWORKSPACE for missing or short scratch, EINVAL for 2^31 or more source positions     */
+/* per cloud and for the arguments the atomic twin rejects.                                      */
+/* ------------------------------------------------------------------------------------------ */
+/* Scratch of a CSR over N destinations of T source positions per cloud (B clouds): the gather,
+ * group and rows twins need (B, N, T), three_interpolate (B, m, 3n). 256-B aligned. */
+size_t b200pci_scatter_workspace_bytes(int B, int N, long long T);
+/* grad_points[b,c,i] = ((g0 + grad_out[b,c,t1]) + grad_out[b,c,t2]) + ...,  t1 < t2 < ... the
+ * positions with idx[b,t] == i (t over npoints, or npoints*nsample for group); g0 the value
+ * grad_points holds: a sequential loop over t. */
+int b200pci_gather_points_grad_det(int b, int c, int n, int npoints, const float *grad_out,
+                                   const int *idx, float *grad_points, void *workspace,
+                                   size_t workspace_bytes, void *stream);
+int b200pci_group_points_grad_det(int b, int c, int n, int npoints, int nsample,
+                                  const float *grad_out, const int *idx, float *grad_points,
+                                  void *workspace, size_t workspace_bytes, void *stream);
+/* grad_points[b,c,k] = g0 + fl(grad_out[b,c,i] * weight[b,i,j]) + ... over the (i, j) with
+ * idx[b,i,j] == k, ascending (i, j), j the slot 0..2 (the repeated slots of three_nn's m < 3 case
+ * in slot order). Scratch b200pci_scatter_workspace_bytes(b, m, 3 n). */
+int b200pci_three_interpolate_grad_det(int b, int c, int n, int m, const float *grad_out,
+                                       const int *idx, const float *weight, float *grad_points,
+                                       void *workspace, size_t workspace_bytes, void *stream);
+/* grad_points[b,i,c] = ((g0 + grad_out[b,t1,c]) + grad_out[b,t2,c]) + ..., t ascending;
+ * grad_points [B,N,C] contiguous, pre-zeroed; idx int64 or int32 [B,T]. */
+int b200pci_index_points_rows_grad_det(int B, int N, long long T, int C, const float *grad_out,
+                                       const void *idx, int idx_is_int64, float *grad_points,
+                                       void *workspace, size_t workspace_bytes, void *stream);
+/* Chamfer, overwriting grad_x / grad_y. Per-point terms as b200pci_chamfer_backward computes
+ * them: w_x = fl(fl(2 g) / fl(B N)), d_x(i) = fl(w_x * fl(x_i - y_{idx_x[i]})), the same for y
+ * with M. grad_x[b,i] = ((0 + d_x(i)) - d_y(j1)) - d_y(j2) - ..., j1 < j2 < ... the points of y
+ * whose nearest x is i; grad_y the mirror image. */
+size_t b200pci_chamfer_backward_det_workspace_bytes(int B, int N, int M);
+int b200pci_chamfer_backward_det(int B, int N, int M, const float *x, const float *y,
+                                 const int *idx_x, const int *idx_y, const float *grad_loss,
+                                 float *grad_x, float *grad_y, void *workspace,
+                                 size_t workspace_bytes, void *stream);
+
+/* ------------------------------------------------------------------------------------------ */
 /* E1-E3: emd_cuda replacements (models/EMD/cuda/emd.cpp:23-27, emd_kernel.cu).                  */
 /* xyz1 [B,n,3], xyz2 [B,m,3] contiguous. match [B,m,n]; temp: scratch of                        */
 /* b200pci_emd_workspace_bytes(B,n,m). Launches on `stream` (the reference uses the legacy       */

@@ -55,6 +55,13 @@ PROTOTYPES = {
     "b200pci_chamfer_forward": (_I, [_I, _I, _I, _P, _L, _L, _L, _P, _L, _L, _L,
                                      _P, _P, _P, _P, _P, _P, _Z, _P]),
     "b200pci_chamfer_backward": (_I, [_I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "b200pci_chamfer_backward_det_workspace_bytes": (_Z, [_I, _I, _I]),
+    "b200pci_chamfer_backward_det": (_I, [_I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _Z, _P]),
+    "b200pci_scatter_workspace_bytes": (_Z, [_I, _I, _c.c_longlong]),
+    "b200pci_gather_points_grad_det": (_I, [_I, _I, _I, _I, _P, _P, _P, _P, _Z, _P]),
+    "b200pci_group_points_grad_det": (_I, [_I, _I, _I, _I, _I, _P, _P, _P, _P, _Z, _P]),
+    "b200pci_three_interpolate_grad_det": (_I, [_I, _I, _I, _I, _P, _P, _P, _P, _P, _Z, _P]),
+    "b200pci_index_points_rows_grad_det": (_I, [_I, _I, _c.c_longlong, _I, _P, _P, _I, _P, _P, _Z, _P]),
     "b200pci_emd_workspace_bytes": (_Z, [_I, _I, _I]),
     "b200pci_emd_approxmatch": (_I, [_I, _I, _I, _P, _P, _P, _P, _Z, _P]),
     "b200pci_emd_matchcost": (_I, [_I, _I, _I, _P, _P, _P, _P, _P, _Z, _P]),

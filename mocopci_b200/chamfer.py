@@ -51,9 +51,16 @@ class _ChamferFunction(Function):
             gx = torch.empty((B, N, 3), dtype=torch.float32, device=x.device)
             gy = torch.empty((B, M, 3), dtype=torch.float32, device=x.device)
             g = grad_loss.reshape(1).contiguous().float()
-            _lib.check(_L.b200pci_chamfer_backward(
-                B, N, M, xc.data_ptr(), yc.data_ptr(), idx_x.data_ptr(), idx_y.data_ptr(),
-                g.data_ptr(), gx.data_ptr(), gy.data_ptr(), _lib.stream_ptr()), "chamfer_backward")
+            if torch.are_deterministic_algorithms_enabled():  # fixed summation order (b200pci.h, _det)
+                ws = _lib.workspace(_L.b200pci_chamfer_backward_det_workspace_bytes(B, N, M), x.device)
+                _lib.check(_L.b200pci_chamfer_backward_det(
+                    B, N, M, xc.data_ptr(), yc.data_ptr(), idx_x.data_ptr(), idx_y.data_ptr(),
+                    g.data_ptr(), gx.data_ptr(), gy.data_ptr(), ws.data_ptr(), ws.numel(),
+                    _lib.stream_ptr()), "chamfer_backward_det")
+            else:
+                _lib.check(_L.b200pci_chamfer_backward(
+                    B, N, M, xc.data_ptr(), yc.data_ptr(), idx_x.data_ptr(), idx_y.data_ptr(),
+                    g.data_ptr(), gx.data_ptr(), gy.data_ptr(), _lib.stream_ptr()), "chamfer_backward")
         return gx, gy
 
 

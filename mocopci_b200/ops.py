@@ -44,7 +44,7 @@ _SPECS = {
 
 class _IndexedCopy(torch.autograd.Function):
     """out = features[..., idx] for the [B, C, N] layout; the gradient is the matching scatter-add
-    (atomics, like the reference's kernels)."""
+    (atomics, like the reference's kernels; in a fixed order under torch's deterministic flag)."""
 
     @staticmethod
     def forward(ctx, kind, features, idx):

@@ -177,10 +177,17 @@ class _IndexRows(torch.autograd.Function):
         g = grad_out.contiguous()
         grad_points = torch.zeros((B, N, C), dtype=torch.float32, device=g.device)
         T = idx_c[0].numel() if B > 0 else 0
+        is64 = 1 if idx_c.dtype == torch.int64 else 0
         with _lib.on_device(g):
-            _lib.check(_L.b200pci_index_points_rows_grad(
-                B, N, T, C, g.data_ptr(), idx_c.data_ptr(), 1 if idx_c.dtype == torch.int64 else 0,
-                grad_points.data_ptr(), _lib.stream_ptr()), "index_points_rows_grad")
+            if torch.are_deterministic_algorithms_enabled():  # fixed summation order (b200pci.h, _det)
+                ws = _lib.workspace(_L.b200pci_scatter_workspace_bytes(B, N, T), g.device)
+                _lib.check(_L.b200pci_index_points_rows_grad_det(
+                    B, N, T, C, g.data_ptr(), idx_c.data_ptr(), is64, grad_points.data_ptr(),
+                    ws.data_ptr(), ws.numel(), _lib.stream_ptr()), "index_points_rows_grad_det")
+            else:
+                _lib.check(_L.b200pci_index_points_rows_grad(
+                    B, N, T, C, g.data_ptr(), idx_c.data_ptr(), is64, grad_points.data_ptr(),
+                    _lib.stream_ptr()), "index_points_rows_grad")
         return grad_points, None
 
 

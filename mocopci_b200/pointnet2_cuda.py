@@ -6,6 +6,10 @@ place on the current CUDA stream, the return value is ignored), so both
 ``pointnet2/pointnet2_utils.py`` and ``models/pointnet2/pointnet2_utils.py`` of the reference run
 unchanged on top of it once ``mocopci_b200.install()`` has registered this module as
 ``sys.modules["pointnet2_cuda"]``. Failures raise ``RuntimeError`` instead of ``exit(-1)``.
+
+Under ``torch.use_deterministic_algorithms(True)`` (``warn_only`` included) the three gradient
+wrappers run the fixed-order ``*_grad_det`` kernels instead of the atomic ones: the gradients are
+then the same bits on every run (include/b200pci.h, "deterministic gradients").
 """
 import torch
 
@@ -49,6 +53,13 @@ def gather_points_wrapper(b, c, n, npoints, points_tensor, idx_tensor, out_tenso
 def gather_points_grad_wrapper(b, c, n, npoints, grad_out_tensor, idx_tensor, grad_points_tensor):
     """sampling.cpp:25-35."""
     with _lib.on_device(grad_out_tensor):
+        if torch.are_deterministic_algorithms_enabled():
+            ws = _lib.workspace(_L.b200pci_scatter_workspace_bytes(b, n, npoints), grad_out_tensor.device)
+            _lib.check(_L.b200pci_gather_points_grad_det(
+                b, c, n, npoints, _f32(grad_out_tensor, "grad_out"), _i32(idx_tensor, "idx"),
+                _f32(grad_points_tensor, "grad_points"), ws.data_ptr(), ws.numel(), _lib.stream_ptr()),
+                "gather_points_grad_det")
+            return 1
         _lib.check(_L.b200pci_gather_points_grad(
             b, c, n, npoints, _f32(grad_out_tensor, "grad_out"), _i32(idx_tensor, "idx"),
             _f32(grad_points_tensor, "grad_points"), _lib.stream_ptr()), "gather_points_grad")
@@ -80,6 +91,13 @@ def group_points_grad_wrapper(b, c, n, npoints, nsample, grad_out_tensor, idx_te
                               grad_points_tensor):
     """group_points.cpp:11-24."""
     with _lib.on_device(grad_out_tensor):
+        if torch.are_deterministic_algorithms_enabled():
+            ws = _lib.workspace(_L.b200pci_scatter_workspace_bytes(b, n, npoints * nsample), grad_out_tensor.device)
+            _lib.check(_L.b200pci_group_points_grad_det(
+                b, c, n, npoints, nsample, _f32(grad_out_tensor, "grad_out"), _i32(idx_tensor, "idx"),
+                _f32(grad_points_tensor, "grad_points"), ws.data_ptr(), ws.numel(), _lib.stream_ptr()),
+                "group_points_grad_det")
+            return 1
         _lib.check(_L.b200pci_group_points_grad(
             b, c, n, npoints, nsample, _f32(grad_out_tensor, "grad_out"), _i32(idx_tensor, "idx"),
             _f32(grad_points_tensor, "grad_points"), _lib.stream_ptr()), "group_points_grad")
@@ -110,6 +128,13 @@ def three_interpolate_grad_wrapper(b, c, n, m, grad_out_tensor, idx_tensor, weig
                                    grad_points_tensor):
     """interpolate.cpp:44-57."""
     with _lib.on_device(grad_out_tensor):
+        if torch.are_deterministic_algorithms_enabled():
+            ws = _lib.workspace(_L.b200pci_scatter_workspace_bytes(b, m, 3 * n), grad_out_tensor.device)
+            _lib.check(_L.b200pci_three_interpolate_grad_det(
+                b, c, n, m, _f32(grad_out_tensor, "grad_out"), _i32(idx_tensor, "idx"),
+                _f32(weight_tensor, "weight"), _f32(grad_points_tensor, "grad_points"), ws.data_ptr(),
+                ws.numel(), _lib.stream_ptr()), "three_interpolate_grad_det")
+            return
         _lib.check(_L.b200pci_three_interpolate_grad(
             b, c, n, m, _f32(grad_out_tensor, "grad_out"), _i32(idx_tensor, "idx"),
             _f32(weight_tensor, "weight"), _f32(grad_points_tensor, "grad_points"),
