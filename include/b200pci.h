@@ -284,6 +284,36 @@ int b200pci_chamfer_backward_det(int B, int N, int M, const float *x, const floa
                                  size_t workspace_bytes, void *stream);
 
 /* ------------------------------------------------------------------------------------------ */
+/* K5: backward of b200pci_knn's distances (any dist_mode; pytorch3d knn_points' backward, the   */
+/* dists of models/pointconv_util.py:910 under autograd). q [B,S,3], r [B,N,3] strided like      */
+/* b200pci_knn; idx int64/int32 [B,S,K] contiguous (b200pci_knn's output); grad_dist [B,S,K]     */
+/* contiguous. grad_q [B,S,3], grad_r [B,N,3] contiguous, OVERWRITTEN.                            */
+/* Arithmetic, for slot (i, k) with j = idx[b,i,k] and each coordinate c:                         */
+/*   d(i,k)_c = fl( fl(2 * grad_dist[b,i,k]) * fl(q[b,i,c] - r[b,j,c]) ), no FMA -- the form of   */
+/*   pytorch3d's KNN backward kernel, 2 * grad_dist * (p1 - p2) (PARITY UNPINNED, as the forward); */
+/*   grad_q[b,i,c] = ((0 + d(i,0)_c) + d(i,1)_c) + ..., k ascending;                              */
+/*   grad_r[b,j,c] = ((0 - d(t1)_c) - d(t2)_c) - ..., over the flat slots t = i*K + k with        */
+/*   idx == j, t ascending (the _det order; the atomic variant adds the same terms in any order).  */
+/* A slot contributes nothing when k >= N (the (inf, 0) padding of the DIRECT modes for K > N) or */
+/* when j is outside [0, N). grad_q has the same bits from both entry points (one thread walks a  */
+/* query's slots in order, no atomics); only grad_r differs.                                      */
+/* Both: EINVAL for negative sizes, null pointers, B > 65535 or S*K >= 2^31; B = 0 or S = N = 0   */
+/* is a no-op. _det: scratch of b200pci_scatter_workspace_bytes(B, N, S*K) (EWORKSPACE when      */
+/* missing or short), the D1 guarantees above (no allocation, no host synchronisation).           */
+/* ------------------------------------------------------------------------------------------ */
+int b200pci_knn_backward(int B, int S, int N, int K,
+                         const float *q, int64_t q_sb, int64_t q_sp, int64_t q_sc,
+                         const float *r, int64_t r_sb, int64_t r_sp, int64_t r_sc,
+                         const void *idx, int idx_is_int64, const float *grad_dist,
+                         float *grad_q, float *grad_r, void *stream);
+int b200pci_knn_backward_det(int B, int S, int N, int K,
+                             const float *q, int64_t q_sb, int64_t q_sp, int64_t q_sc,
+                             const float *r, int64_t r_sb, int64_t r_sp, int64_t r_sc,
+                             const void *idx, int idx_is_int64, const float *grad_dist,
+                             float *grad_q, float *grad_r, void *workspace,
+                             size_t workspace_bytes, void *stream);
+
+/* ------------------------------------------------------------------------------------------ */
 /* E1-E3: emd_cuda replacements (models/EMD/cuda/emd.cpp:23-27, emd_kernel.cu).                  */
 /* xyz1 [B,n,3], xyz2 [B,m,3] contiguous. match [B,m,n]; temp: scratch of                        */
 /* b200pci_emd_workspace_bytes(B,n,m). Launches on `stream` (the reference uses the legacy       */

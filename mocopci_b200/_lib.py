@@ -62,6 +62,9 @@ PROTOTYPES = {
     "b200pci_group_points_grad_det": (_I, [_I, _I, _I, _I, _I, _P, _P, _P, _P, _Z, _P]),
     "b200pci_three_interpolate_grad_det": (_I, [_I, _I, _I, _I, _P, _P, _P, _P, _P, _Z, _P]),
     "b200pci_index_points_rows_grad_det": (_I, [_I, _I, _c.c_longlong, _I, _P, _P, _I, _P, _P, _Z, _P]),
+    "b200pci_knn_backward": (_I, [_I, _I, _I, _I, _P, _L, _L, _L, _P, _L, _L, _L, _P, _I, _P, _P, _P, _P]),
+    "b200pci_knn_backward_det": (_I, [_I, _I, _I, _I, _P, _L, _L, _L, _P, _L, _L, _L, _P, _I, _P, _P, _P,
+                                      _P, _Z, _P]),
     "b200pci_emd_workspace_bytes": (_Z, [_I, _I, _I]),
     "b200pci_emd_approxmatch": (_I, [_I, _I, _I, _P, _P, _P, _P, _Z, _P]),
     "b200pci_emd_matchcost": (_I, [_I, _I, _I, _P, _P, _P, _P, _P, _Z, _P]),

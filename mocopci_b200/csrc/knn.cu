@@ -7,6 +7,7 @@
 #include "nbr_two_pass.cuh"
 #include "nbr_scan_eval.cuh"
 #include "nbr_scan_tc.cuh"
+#include "knn_grad.cuh"
 
 extern int g_fps_single_cta;  // fps.cu (test hook)
 int b200pci_gather_debug_set(int key, double value);  // gather.cu (developer hooks 15, 16)
@@ -1229,6 +1230,22 @@ __global__ void chamfer_backward_kernel(int B, int N, int M, const float *__rest
     }
 }
 
+// Backward of b200pci_knn's distances: thread per query (knn_grad.cuh); grad_r (pre-zeroed) gets
+// -d(i,k) of every live slot through atomics, in no particular order.
+template <typename I>
+__global__ void __launch_bounds__(256)
+    knn_backward_kernel(KnnGradArgs a, const I *__restrict__ idx, float *__restrict__ grad_r) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    const int b = blockIdx.y;
+    if (i >= a.S) return;
+    float *gr = grad_r + (size_t)b * a.N * 3;
+    knn_grad_query(a, b, i, idx, [&](long long j, float dx, float dy, float dz) {
+        atomicAdd(gr + j * 3, -dx);
+        atomicAdd(gr + j * 3 + 1, -dy);
+        atomicAdd(gr + j * 3 + 2, -dz);
+    });
+}
+
 }  // namespace b200pci
 
 using namespace b200pci;
@@ -1598,6 +1615,31 @@ extern "C" int b200pci_chamfer_backward(int B, int N, int M, const float *x, con
             B, N, M, x, y, idx_x, idx_y, grad_loss, grad_x, grad_y, 1);
         B200PCI_LAUNCH_CHECK("chamfer_backward_kernel");
     }
+    return B200PCI_OK;
+}
+
+extern "C" int b200pci_knn_backward(int B, int S, int N, int K, const float *q, int64_t q_sb, int64_t q_sp,
+                                    int64_t q_sc, const float *r, int64_t r_sb, int64_t r_sp, int64_t r_sc,
+                                    const void *idx, int idx_is_int64, const float *grad_dist, float *grad_q,
+                                    float *grad_r, void *stream) {
+    cudaStream_t st = (cudaStream_t)stream;
+    bool nothing;
+    if (int rc = knn_grad_check(B, S, N, K, q, r, idx, grad_dist, grad_q, grad_r, "knn_backward", &nothing))
+        return rc;
+    if (nothing) return B200PCI_OK;
+    B200PCI_CUDA(cudaMemsetAsync(grad_r, 0, (size_t)B * N * 3 * sizeof(float), st));
+    if (S == 0) return B200PCI_OK;
+    if (K == 0 || N == 0) {  // no live slot
+        B200PCI_CUDA(cudaMemsetAsync(grad_q, 0, (size_t)B * S * 3 * sizeof(float), st));
+        return B200PCI_OK;
+    }
+    const KnnGradArgs a{S, N, K, q, q_sb, q_sp, q_sc, r, r_sb, r_sp, r_sc, grad_dist, grad_q};
+    const dim3 grid(ceil_div(S, 256), B);
+    if (idx_is_int64)
+        knn_backward_kernel<long long><<<grid, 256, 0, st>>>(a, reinterpret_cast<const long long *>(idx), grad_r);
+    else
+        knn_backward_kernel<int><<<grid, 256, 0, st>>>(a, reinterpret_cast<const int *>(idx), grad_r);
+    B200PCI_LAUNCH_CHECK("knn_backward_kernel");
     return B200PCI_OK;
 }
 

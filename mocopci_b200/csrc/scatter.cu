@@ -1,5 +1,5 @@
 // Deterministic (fixed-order) versions of the scatter-add gradients: gather / group, three_interpolate,
-// the [B,N,C] row gathers and Chamfer. The atomic kernels (gather.cu, knn.cu) add the contributions
+// the [B,N,C] row gathers, Chamfer and the K-NN distances. The atomic kernels (gather.cu, knn.cu) add the contributions
 // to one destination in whatever order the threads arrive, so the last bits of a gradient change
 // from run to run. Here each destination sums its contributions sequentially in FP32, in ascending
 // source position, every product rounded before it is added (include/b200pci.h, "_det").
@@ -15,6 +15,7 @@
 #include <algorithm>
 
 #include "common.cuh"
+#include "knn_grad.cuh"
 
 namespace b200pci {
 
@@ -394,6 +395,48 @@ __global__ void __launch_bounds__(SC_THREADS)
     dst[2] = az;
 }
 
+// K-NN distances: grad_q by one thread per query (knn_grad.cuh, the atomic kernel's own pass
+// without the scatter), grad_r by one thread per ref over its bucket of slots t = i*K + k:
+// grad_r[b,j] = ((0 - d(t1)) - d(t2)) - ..., t ascending; padded slots (k >= N) are skipped.
+template <typename I>
+__global__ void __launch_bounds__(SC_THREADS) knn_grad_q_det_kernel(KnnGradArgs a, const I *__restrict__ idx) {
+    const int i = blockIdx.x * SC_THREADS + threadIdx.x;
+    const int b = blockIdx.y;
+    if (i >= a.S) return;
+    knn_grad_query(a, b, i, idx, [](long long, float, float, float) {});
+}
+
+__global__ void __launch_bounds__(SC_THREADS)
+    knn_grad_r_det_kernel(KnnGradArgs a, const int *__restrict__ offsets, const int *__restrict__ list,
+                          float *__restrict__ grad_r) {
+    const int j = blockIdx.x * SC_THREADS + threadIdx.x;
+    const int b = blockIdx.y;
+    if (j >= a.N) return;
+    const long long T = (long long)a.S * a.K;
+    const float *rj = a.r + b * a.r_sb + j * a.r_sp;
+    const float rx = __ldg(rj), ry = __ldg(rj + a.r_sc), rz = __ldg(rj + 2 * a.r_sc);
+    const int beg = offsets[(size_t)b * (a.N + 1) + j], end = offsets[(size_t)b * (a.N + 1) + j + 1];
+    const int *l = list + (size_t)b * T;
+    const float *gd = a.grad_dist + (size_t)b * T;
+    const float *qb = a.q + b * a.q_sb;
+    float ax = 0.f, ay = 0.f, az = 0.f;
+#pragma unroll 4
+    for (int p = beg; p < end; ++p) {
+        const int t = __ldg(l + p);
+        const int i = t / a.K, k = t - i * a.K;
+        if (k >= a.N) continue;
+        const float g2 = __fmul_rn(2.f, __ldg(gd + t));
+        const float *qi = qb + i * a.q_sp;
+        ax = __fsub_rn(ax, __fmul_rn(g2, __fsub_rn(__ldg(qi), rx)));
+        ay = __fsub_rn(ay, __fmul_rn(g2, __fsub_rn(__ldg(qi + a.q_sc), ry)));
+        az = __fsub_rn(az, __fmul_rn(g2, __fsub_rn(__ldg(qi + 2 * a.q_sc), rz)));
+    }
+    float *dst = grad_r + ((size_t)b * a.N + j) * 3;
+    dst[0] = ax;
+    dst[1] = ay;
+    dst[2] = az;
+}
+
 static int check_ws(void *workspace, size_t have, size_t need, const char *what) {
     if (!workspace || have < need) {
         set_error("%s: workspace of %zu bytes required, got %zu", what, need, have);
@@ -523,5 +566,38 @@ extern "C" int b200pci_chamfer_backward_det(int B, int N, int M, const float *x,
     chamfer_grad_det_kernel<<<dim3(ceil_div(M, SC_THREADS), B), SC_THREADS, 0, st>>>(
         B, M, N, y, x, idx_y, grad_loss, by_y.offsets, by_y.list, grad_y);
     B200PCI_LAUNCH_CHECK("chamfer_grad_det_kernel");
+    return B200PCI_OK;
+}
+
+extern "C" int b200pci_knn_backward_det(int B, int S, int N, int K, const float *q, int64_t q_sb, int64_t q_sp,
+                                        int64_t q_sc, const float *r, int64_t r_sb, int64_t r_sp, int64_t r_sc,
+                                        const void *idx, int idx_is_int64, const float *grad_dist, float *grad_q,
+                                        float *grad_r, void *workspace, size_t workspace_bytes, void *stream) {
+    const char *what = "knn_backward_det";
+    cudaStream_t st = (cudaStream_t)stream;
+    bool nothing;
+    if (int rc = knn_grad_check(B, S, N, K, q, r, idx, grad_dist, grad_q, grad_r, what, &nothing)) return rc;
+    if (nothing) return B200PCI_OK;
+    const long long T = (long long)S * K;
+    if (int rc = check_ws(workspace, workspace_bytes, csr_bytes(B, N, T), what)) return rc;
+    if (T == 0 || N == 0) {  // no live slot: both gradients are zero
+        B200PCI_CUDA(cudaMemsetAsync(grad_q, 0, (size_t)B * S * 3 * sizeof(float), st));
+        B200PCI_CUDA(cudaMemsetAsync(grad_r, 0, (size_t)B * N * 3 * sizeof(float), st));
+        return B200PCI_OK;
+    }
+    const Csr csr = csr_carve(workspace, B, N, T);
+    int rc = idx_is_int64 ? csr_build<long long>(B, N, T, reinterpret_cast<const long long *>(idx), csr, st)
+                          : csr_build<int>(B, N, T, reinterpret_cast<const int *>(idx), csr, st);
+    if (rc) return rc;
+    const KnnGradArgs a{S, N, K, q, q_sb, q_sp, q_sc, r, r_sb, r_sp, r_sc, grad_dist, grad_q};
+    if (idx_is_int64)
+        knn_grad_q_det_kernel<long long><<<dim3(ceil_div(S, SC_THREADS), B), SC_THREADS, 0, st>>>(
+            a, reinterpret_cast<const long long *>(idx));
+    else
+        knn_grad_q_det_kernel<int><<<dim3(ceil_div(S, SC_THREADS), B), SC_THREADS, 0, st>>>(
+            a, reinterpret_cast<const int *>(idx));
+    B200PCI_LAUNCH_CHECK("knn_grad_q_det_kernel");
+    knn_grad_r_det_kernel<<<dim3(ceil_div(N, SC_THREADS), B), SC_THREADS, 0, st>>>(a, csr.offsets, csr.list, grad_r);
+    B200PCI_LAUNCH_CHECK("knn_grad_r_det_kernel");
     return B200PCI_OK;
 }
