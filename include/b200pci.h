@@ -361,7 +361,9 @@ int b200pci_probe_fp32(int packed, int iters, float *sink, double *flops, void *
  *   20  0 = thread t of the top-k kernel takes query t (1 = queries handed out by list length)
  *   19  lanes per row of the forward-only EMD sweeps: 4, 8, 16 (default), 32
  *   15 / 16  three_interpolate: point slices of the quad kernel (0 = automatic) / 1 = rows kernel
- * b200pci_debug_get(key): 3 = accumulated ms of the timed launches, 4 = their number. */
+ * b200pci_debug_get(key): 3 = accumulated ms of the timed launches, 4 = their number;
+ *    5 / 6 = flagged tiles / flagged queries of the calling thread's last two-pass KNN call
+ *    (synchronises the device; -1 if this thread has made none). */
 int b200pci_debug_set(int key, double value);
 double b200pci_debug_get(int key);
 

@@ -593,7 +593,9 @@ static int g_tau_tc = 1;  // key 9 (tests): 0 = FP32-pipe threshold pre-pass (kn
 // ~12 m boxes against bounds of ~1 m, so a 256-query CTA still keeps 58 % of the tiles, the sort
 // costs 0.2 ms per call, and spatially concentrated candidates overflow the per-split lists.
 static int g_sort = 0;
-static const int *g_last_fail = nullptr;  // developer: redo counters of the last two-pass call (debug_get 5 / 6)
+// developer: redo counters of the calling thread's last two-pass call (debug_get 5 / 6); every
+// two-pass call writes it, so it is per thread like the library's other state
+static thread_local const int *g_last_fail = nullptr;
 static int g_use_tc = 1;  // key 8 (tests): 0 = FP32-pipe filter (knn_scan_eval_kernel) instead of the tensor-core one
 // key 3: time the dominant kernel of every b200pci_knn call (knn_scan_kernel on the two-pass path,
 // knn_kernel otherwise) with CUDA events on the launching stream; b200pci_debug_get(3) -> accumulated ms, (4) -> number of timed launches.
