@@ -314,6 +314,42 @@ int b200pci_knn_backward_det(int B, int S, int N, int K,
                              size_t workspace_bytes, void *stream);
 
 /* ------------------------------------------------------------------------------------------ */
+/* P1 / P2: pytorch3d.ops.ball_query and pytorch3d.ops.sample_farthest_points (0.7.5, PARITY     */
+/* UNPINNED as for knn_points: the contract below is this library's own). Ragged batches: the    */
+/* per-cloud lengths are int64 [B] DEVICE arrays, read by the kernels and clamped to [0, P]      */
+/* (NULL: every cloud has P points). Neither call allocates, needs scratch or synchronises with  */
+/* the host; both are graph capturable and launch one kernel on `stream`.                        */
+/* ------------------------------------------------------------------------------------------ */
+/* P1: p1 [B,P1,3], p2 [B,P2,3] float32 through element strides (like b200pci_knn). For query    */
+/* i < lengths1[b], the slots of idx[b,i,:] hold, in ascending j, the first K refs j < lengths2[b] */
+/* with d2 < r2 (strict), d2 = fma(dz,dz,fma(dy,dy,dx*dx)), d = p1[b,i] - p2[b,j] (DIST_DIRECT_XYZ) */
+/* and r2 = radius * radius rounded in FP32; dists holds those d2. Slots past the hits, and every   */
+/* slot of a query i >= lengths1[b], are idx = -1, dists = 0. idx int64 [B,P1,K], dists float32    */
+/* [B,P1,K], nn (nullable) float32 [B,P1,K,3] = p2[b, idx] row by row (zeros where idx = -1).     */
+/* Every output element is written. EINVAL: negative sizes, K < 1, radius < 0 or NaN, null        */
+/* pointers, B > 65535. B = 0 or P1 = 0 is a no-op. The distance backward is b200pci_knn_backward */
+/* (_det) with this idx as is: -1 slots contribute nothing, and a query has at most P2 hits, so    */
+/* none sits in a slot k >= P2.                                                                   */
+/* ------------------------------------------------------------------------------------------ */
+int b200pci_ball_query_p3d(int B, int P1, int P2, int K, float radius,
+                           const float *p1, int64_t p1_sb, int64_t p1_sp, int64_t p1_sc,
+                           const float *p2, int64_t p2_sb, int64_t p2_sp, int64_t p2_sc,
+                           const int64_t *lengths1, const int64_t *lengths2,
+                           int64_t *idx, float *dists, float *nn, void *stream);
+/* P2: points [B,P,3] float32 through element strides. Per cloud n = lengths[b] points and         */
+/* m = min(K[b], n) picks (K: int64 [B] device array, values clamped to [0, M]; NULL: M for every */
+/* cloud). idx[b,0] = start[b] (int64 [B] device array clamped to [0, n-1]; NULL: 0); pick t > 0   */
+/* is the argmax over j < n of the running minimum, over the earlier picks, of                   */
+/* d2 = fma(dz,dz,fma(dy,dy,dx*dx)) (the minimum starts at +inf); among equal values the LOWEST   */
+/* index wins (b200pci_furthest_point_sampling keeps the reference's bit-reversed thread order    */
+/* instead). Picks m..M-1 are -1. idx int64 [B,M]; selected (nullable) float32 [B,M,3] = the      */
+/* picked points' rows, zeros for -1. EINVAL: negative sizes, null pointers, P > 131072,          */
+/* B > 2^27. B = 0 or M = 0 is a no-op.                                                            */
+int b200pci_fps_p3d(int B, int P, int M, const float *points, int64_t p_sb, int64_t p_sp,
+                    int64_t p_sc, const int64_t *lengths, const int64_t *K, const int64_t *start,
+                    int64_t *idx, float *selected, void *stream);
+
+/* ------------------------------------------------------------------------------------------ */
 /* E1-E3: emd_cuda replacements (models/EMD/cuda/emd.cpp:23-27, emd_kernel.cu).                  */
 /* xyz1 [B,n,3], xyz2 [B,m,3] contiguous. match [B,m,n]; temp: scratch of                        */
 /* b200pci_emd_workspace_bytes(B,n,m). Launches on `stream` (the reference uses the legacy       */

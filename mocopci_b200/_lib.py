@@ -65,6 +65,8 @@ PROTOTYPES = {
     "b200pci_knn_backward": (_I, [_I, _I, _I, _I, _P, _L, _L, _L, _P, _L, _L, _L, _P, _I, _P, _P, _P, _P]),
     "b200pci_knn_backward_det": (_I, [_I, _I, _I, _I, _P, _L, _L, _L, _P, _L, _L, _L, _P, _I, _P, _P, _P,
                                       _P, _Z, _P]),
+    "b200pci_ball_query_p3d": (_I, [_I, _I, _I, _I, _F, _P, _L, _L, _L, _P, _L, _L, _L, _P, _P, _P, _P, _P, _P]),
+    "b200pci_fps_p3d": (_I, [_I, _I, _I, _P, _L, _L, _L, _P, _P, _P, _P, _P, _P]),
     "b200pci_emd_workspace_bytes": (_Z, [_I, _I, _I]),
     "b200pci_emd_approxmatch": (_I, [_I, _I, _I, _P, _P, _P, _P, _Z, _P]),
     "b200pci_emd_matchcost": (_I, [_I, _I, _I, _P, _P, _P, _P, _P, _Z, _P]),

@@ -20,7 +20,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libb200pci.so")
-SOURCES = ["common.cu", "knn.cu", "fps.cu", "gather.cu", "emd.cu", "probe.cu", "cosine.cu", "scatter.cu"]
+SOURCES = ["common.cu", "knn.cu", "fps.cu", "gather.cu", "emd.cu", "probe.cu", "cosine.cu", "scatter.cu",
+           "ball_p3d.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
          "-Xcompiler", "-fPIC"] + os.environ.get("B200PCI_EXTRA_NVCC_FLAGS", "").split()

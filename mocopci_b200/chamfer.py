@@ -13,7 +13,8 @@ through b200pci_knn_backward (b200pci_knn_backward_det under torch.use_determini
 ``knn`` (return_nn) through the row-gather backward. ``chamfer_distance`` with default arguments runs
 the fused Chamfer kernels; its other reduction options, per-cloud weights and the one-way form are
 composed in torch from two differentiable ``knn_points(K=1)`` calls, as pytorch3d 0.7.5 does. Ragged
-batches (lengths), normals and the L1 norm are not implemented.
+batches (lengths), normals and the L1 norm are not implemented here; pytorch3d's ``ball_query`` and
+``sample_farthest_points``, which do take per-cloud lengths, are in p3d_ops.py.
 """
 from collections import namedtuple
 

@@ -293,6 +293,171 @@ __global__ void __launch_bounds__(CT, 1)
     cluster.sync();  // no CTA exits while a peer may still write into it
 }
 
+// ---- pytorch3d form (b200pci_fps_p3d) ------------------------------------------------------------
+// The cluster scheme above with pytorch3d's sample_farthest_points rules: per cloud n = lengths[b]
+// points and m = min(K[b], n) picks (both read here, on the device), the first pick start[b], the
+// running minimum starts at +inf (no temp buffer), d = fma(dz,dz,fma(dy,dy,dx*dx)), and the tie key
+// is the point index itself (~k: the lowest index wins). Picks m..M-1 are written as -1 with zero
+// rows. Points are read through element strides; the mirror holds them as [n][3].
+constexpr int FPS3_CS = 8, FPS3_CT = 512;
+
+struct Fps3Args {
+    int N, M, chunk;
+    const float *xyz;
+    long long sb, sp, sc;
+    const long long *lengths, *K, *start;  // [B] each, nullable
+    long long *idx;                        // [B, M]
+    float *sel;                            // [B, M, 3], nullable
+};
+
+template <int PT, bool MIRROR>
+__global__ void __launch_bounds__(FPS3_CT, 1) fps_p3d_cluster_kernel(Fps3Args a) {
+    constexpr int CS = FPS3_CS, CT = FPS3_CT;
+    cg::cluster_group cluster = cg::this_cluster();
+    const unsigned rank = cluster.block_rank();
+    const int cloud = blockIdx.x / CS;
+    extern __shared__ float sxyz[];  // the cloud's n points, [n][3] (MIRROR)
+    __shared__ unsigned long long part[CT / 32];
+    __shared__ __align__(8) unsigned long long rec[2][CS];
+    __shared__ __align__(8) uint64_t bar[2];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const float *xyz = a.xyz + cloud * a.sb;
+    const long long nl = a.lengths ? a.lengths[cloud] : a.N;
+    const int n = (int)(nl < 0 ? 0 : (nl > a.N ? a.N : nl));
+    const long long kl = a.K ? a.K[cloud] : a.M;
+    const int m = (int)min((long long)n, kl < 0 ? 0 : (kl > a.M ? a.M : kl));
+    long long *idx = a.idx + (size_t)cloud * a.M;
+    float *sel = a.sel ? a.sel + (size_t)cloud * a.M * 3 : nullptr;
+    const int k0 = rank * a.chunk, k1 = min(n, k0 + a.chunk);
+
+    if (rank == 0)
+        for (int j = m + tid; j < a.M; j += CT) {
+            idx[j] = -1;
+            if (sel) sel[3 * j] = sel[3 * j + 1] = sel[3 * j + 2] = 0.f;
+        }
+    float px[PT], py[PT], pz[PT], pt[PT];
+    uint32_t plow[PT];  // ~index of the point (0 = no point)
+#pragma unroll
+    for (int i = 0; i < PT; ++i) {
+        const int k = k0 + tid + i * CT;
+        if (k < k1) {
+            const float *p = xyz + k * a.sp;
+            px[i] = p[0];
+            py[i] = p[a.sc];
+            pz[i] = p[2 * a.sc];
+            pt[i] = __int_as_float(0x7f800000);
+            plow[i] = ~(uint32_t)k;
+        } else {
+            px[i] = py[i] = pz[i] = 0.f;
+            pt[i] = -1.f;
+            plow[i] = 0u;
+        }
+    }
+    if (MIRROR)
+        for (int k = tid; k < n; k += CT) {
+            const float *p = xyz + k * a.sp;
+            sxyz[3 * k] = p[0];
+            sxyz[3 * k + 1] = p[a.sc];
+            sxyz[3 * k + 2] = p[2 * a.sc];
+        }
+    if (tid == 0) {
+        mbar_init(&bar[0], 1);
+        mbar_init(&bar[1], 1);
+        mbar_fence_init();
+    }
+    int old = 0;
+    float x1 = 0.f, y1 = 0.f, z1 = 0.f;
+    if (m > 0) {
+        const long long s = a.start ? a.start[cloud] : 0;
+        old = (int)(s < 0 ? 0 : (s >= n ? n - 1 : s));
+        const float *p = xyz + old * a.sp;
+        x1 = p[0];
+        y1 = p[a.sc];
+        z1 = p[2 * a.sc];
+        if (rank == 0 && tid == 0) {
+            idx[0] = old;
+            if (sel) sel[0] = x1, sel[1] = y1, sel[2] = z1;
+        }
+    }
+    __syncthreads();
+    cluster.sync();  // every CTA's barriers are initialised before the first remote store
+
+    for (int j = 1; j < m; ++j) {
+        const int s = j & 1;
+        if (tid == 0) mbar_arrive_expect_tx(&bar[s], CS * sizeof(unsigned long long));
+        uint32_t bd = 0u, bl = 0u;  // best (distance bits, ~index) of this thread
+#pragma unroll
+        for (int i = 0; i < PT; ++i) {
+            const float dx = __fsub_rn(px[i], x1), dy = __fsub_rn(py[i], y1), dz = __fsub_rn(pz[i], z1);
+            const float d = __fmaf_rn(dz, dz, __fmaf_rn(dy, dy, __fmul_rn(dx, dx)));
+            const float d2 = fminf(d, pt[i]);
+            pt[i] = d2;
+            const uint32_t db = (d2 >= 0.f) ? __float_as_uint(d2) : 0u;  // -1 marks "no point"
+            const bool better = (db > bd) || (db == bd && plow[i] > bl);
+            bd = better ? db : bd;
+            bl = better ? plow[i] : bl;
+        }
+        const unsigned long long wk = warp_argmax_key(bd, bl);
+        if (lane == 0) part[warp] = wk;
+        __syncthreads();
+        if (warp == 0) {
+            const unsigned long long v = (lane < CT / 32) ? part[lane] : 0ull;
+            const unsigned long long ck = warp_argmax_key((uint32_t)(v >> 32), (uint32_t)v);
+            if (lane < CS)
+                st_async_u64(mapa_u32(smem_u32(&rec[s][rank]), lane), ck,
+                             mapa_u32(smem_u32(&bar[s]), lane));
+        }
+        while (!mbar_try_wait_cluster(&bar[s], ((j - 1) >> 1) & 1)) {
+        }
+        unsigned long long best = 0ull;
+#pragma unroll
+        for (int r = 0; r < CS; ++r) {
+            const unsigned long long c = rec[s][r];
+            best = c > best ? c : best;
+        }
+        old = (int)~(uint32_t)best;
+        if (MIRROR) {
+            x1 = sxyz[old * 3 + 0];
+            y1 = sxyz[old * 3 + 1];
+            z1 = sxyz[old * 3 + 2];
+        } else {
+            const float *p = xyz + old * a.sp;
+            x1 = __ldg(p);
+            y1 = __ldg(p + a.sc);
+            z1 = __ldg(p + 2 * a.sc);
+        }
+        if (rank == 0 && tid == 0) {
+            idx[j] = old;
+            if (sel) sel[3 * j] = x1, sel[3 * j + 1] = y1, sel[3 * j + 2] = z1;
+        }
+    }
+    cluster.sync();  // no CTA exits while a peer may still write into it
+}
+
+template <int PT>
+static int launch_fps_p3d(int b, const Fps3Args &a, cudaStream_t st) {
+    const size_t smem = (size_t)a.N * 3 * sizeof(float);
+    const bool mirror = smem <= 200 * 1024;
+    auto kern = mirror ? fps_p3d_cluster_kernel<PT, true> : fps_p3d_cluster_kernel<PT, false>;
+    const size_t dyn = mirror ? smem : 0;
+    if (dyn > 40 * 1024)
+        B200PCI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(b * FPS3_CS);
+    cfg.blockDim = dim3(FPS3_CT);
+    cfg.dynamicSmemBytes = dyn;
+    cfg.stream = st;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = FPS3_CS;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    B200PCI_CUDA(cudaLaunchKernelEx(&cfg, kern, a));
+    return B200PCI_OK;
+}
+
 template <int PT, bool MIRROR, int CS, int CT>
 static int launch_fps_cluster_impl(int b, int n, int m, int chunk, const float *xyz, float *temp,
                                    int *idx, FpsGeom g, cudaStream_t st) {
@@ -407,4 +572,35 @@ extern "C" int b200pci_furthest_point_sampling(int b, int n, int m, const float 
     if (need <= 16) return launch_fps<16>(b, n, m, xyz, temp, idx, g, threads, st);
     if (need <= 32) return launch_fps<32>(b, n, m, xyz, temp, idx, g, threads, st);
     return launch_fps<0>(b, n, m, xyz, temp, idx, g, threads, st);
+}
+
+extern "C" int b200pci_fps_p3d(int B, int P, int M, const float *points, int64_t p_sb, int64_t p_sp,
+                               int64_t p_sc, const int64_t *lengths, const int64_t *K,
+                               const int64_t *start, int64_t *idx, float *selected, void *stream) {
+    B200PCI_CHECK_ARG(B >= 0 && P >= 0 && M >= 0, "fps_p3d: negative size");
+    if (B == 0 || M == 0) return B200PCI_OK;
+    B200PCI_CHECK_ARG(idx && (points || P == 0), "fps_p3d: null pointer");
+    B200PCI_CHECK_ARG(P <= FPS3_CS * FPS3_CT * 32, "fps_p3d: more than %d points per cloud",
+                      FPS3_CS * FPS3_CT * 32);
+    B200PCI_CHECK_ARG(B <= (1 << 27), "fps_p3d: batch too large");
+    Fps3Args a;
+    a.N = P;
+    a.M = M;
+    a.chunk = (P + FPS3_CS - 1) / FPS3_CS;
+    a.xyz = points;
+    a.sb = p_sb;
+    a.sp = p_sp;
+    a.sc = p_sc;
+    a.lengths = reinterpret_cast<const long long *>(lengths);
+    a.K = reinterpret_cast<const long long *>(K);
+    a.start = reinterpret_cast<const long long *>(start);
+    a.idx = reinterpret_cast<long long *>(idx);
+    a.sel = selected;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int need = (a.chunk + FPS3_CT - 1) / FPS3_CT;
+    if (need <= 2) return launch_fps_p3d<2>(B, a, st);
+    if (need <= 4) return launch_fps_p3d<4>(B, a, st);
+    if (need <= 8) return launch_fps_p3d<8>(B, a, st);
+    if (need <= 16) return launch_fps_p3d<16>(B, a, st);
+    return launch_fps_p3d<32>(B, a, st);
 }

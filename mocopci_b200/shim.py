@@ -9,7 +9,8 @@
      own autograd wrappers run unchanged on the B200 kernels;
   2. if pytorch3d is absent, registers ``pytorch3d.loss.chamfer_distance``,
      ``pytorch3d.ops.knn_points`` and ``pytorch3d.ops.knn_gather`` (models/utils.py:8,
-     models/pointconv_util.py:9, models/layers.py:18); if timm is absent, a minimal
+     models/pointconv_util.py:9, models/layers.py:18), plus ``pytorch3d.ops.ball_query`` and
+     ``pytorch3d.ops.sample_farthest_points`` (p3d_ops.py); if timm is absent, a minimal
      ``timm.models.layers`` (DropPath, to_2tuple, trunc_normal_; models/m_models/mocopci.py:4);
   3. re-points the pure-torch helpers of the hot path -- ``knn_point`` (square_distance + topk),
      ``knn_point_cosine`` (cosine_distance + topk), ``index_points_group``, ``index_points_gather``
@@ -328,13 +329,15 @@ class _PostImportPatcher(importlib.abc.MetaPathFinder):
 
 
 def _pytorch3d_shim():
-    from . import chamfer
+    from . import chamfer, p3d_ops
     p3d = types.ModuleType("pytorch3d")
     loss = types.ModuleType("pytorch3d.loss")
     ops = types.ModuleType("pytorch3d.ops")
     loss.chamfer_distance = chamfer.chamfer_distance
     ops.knn_points = chamfer.knn_points
     ops.knn_gather = chamfer.knn_gather
+    ops.ball_query = p3d_ops.ball_query
+    ops.sample_farthest_points = p3d_ops.sample_farthest_points
     p3d.loss, p3d.ops = loss, ops
     p3d.__b200pci_shim__ = True
     return {"pytorch3d": p3d, "pytorch3d.loss": loss, "pytorch3d.ops": ops}
