@@ -386,17 +386,15 @@ int b200pci_probe_fp32(int packed, int iters, float *sink, double *flops, void *
  *    5  1 = force the single-CTA FPS kernel (0)
  *    6  1 = send every ball query through the exact redo kernel (0)
  *    7  pair count from which k <= 4 takes the two-pass path (0 = default 2^25)
- *    8  0 = FP32-pipe filter (knn_scan_eval_kernel) instead of the tensor-core scan (1)
- *    9  0 = FP32-pipe threshold pre-pass instead of the tensor-core one (1)
  *   11  R of the estimated bound (0 = default by k)
  *   12 / 13  ref count / pair count from which k = 5..32 takes the two-pass path (0 = defaults)
  *   14  number of (equal) chunks of b200pci_knn_host's copy pipeline (0 = default: tapered schedule)
- *   17  1 = experimental: Morton-sort the clouds and skip ref tiles that cannot hold a candidate (0)
  *   18  0 = thread-per-query top-k kernel even for small launches (1 = one thread per (query, split group)
  *       for launches of fewer than two CTAs per SM, 2 = whenever the refs are split)
  *   20  0 = thread t of the top-k kernel takes query t (1 = queries handed out by list length)
  *   19  lanes per row of the forward-only EMD sweeps: 4, 8, 16 (default), 32
  *   15 / 16  three_interpolate: point slices of the quad kernel (0 = automatic) / 1 = rows kernel
+ *   any other key: B200PCI_EINVAL, nothing changed
  * b200pci_debug_get(key): 3 = accumulated ms of the timed launches, 4 = their number;
  *    5 / 6 = flagged tiles / flagged queries of the calling thread's last two-pass KNN call
  *    (synchronises the device; -1 if this thread has made none). */

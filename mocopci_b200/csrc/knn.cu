@@ -5,7 +5,7 @@
 
 #include "nbr_engine.cuh"
 #include "nbr_two_pass.cuh"
-#include "nbr_scan_eval.cuh"
+#include "nbr_topk.cuh"
 #include "nbr_scan_tc.cuh"
 #include "knn_grad.cuh"
 
@@ -45,17 +45,11 @@ __global__ void __launch_bounds__(KNN_CW * 32, KNN_CTAS_PER_SM) knn_scan_kernel(
     nbr_scan<KNN_CW, KNN_STAGES>(p);
 }
 
+// the two-pass KNN's scan: filter on the tensor cores, exact evaluation of what it flags (nbr_scan_tc.cuh)
 template <int MODE>
-__global__ void __launch_bounds__(32, KNN_CTAS_PER_SM)
-    knn_scan_eval_kernel(NbrParams p, ScanEvalParams ep) {
-    nbr_scan_eval<MODE, KNN_STAGES>(p, ep);
-}
-
-// the same pass with the filter on the tensor cores (nbr_scan_tc.cuh)
-template <int MODE, bool CULL>
 __global__ void __launch_bounds__(TC_THREADS, TC_UNITS == 1 ? 2 : 1)
-    knn_scan_tc_kernel(NbrParams p, ScanEvalParams ep, const float *ws_tc) {
-    nbr_scan_tc<MODE, CULL>(p, ep, ws_tc);
+    knn_scan_tc_kernel(NbrParams p, ScanEvalParams ep) {
+    nbr_scan_tc<MODE>(p, ep);
 }
 
 template <int RMAX>
@@ -88,7 +82,6 @@ struct MidArgs {
     long long r_sb, r_sp, r_sc;
     int swap_xy;  // DIST_DIRECT_XYZ: first and second coordinate change places (see NbrParams::q_ox)
     int q_xzy, r_xzy;  // norm order of the expanded form (see NbrParams)
-    const int *qperm;  // redo mode on sorted clouds: processed query row -> original row (else null)
     void *idx;
     int idx_is_int64;
     float *dist;
@@ -232,7 +225,7 @@ __device__ __forceinline__ void knn_mid_tile(const MidArgs &a, int b, int tile) 
             merge_sorted16(C);
         }
     }
-    const size_t qrow = (size_t)b * S + (a.qperm ? a.qperm[(size_t)b * S + qi] : qi);
+    const size_t qrow = (size_t)b * S + qi;
 #pragma unroll
     for (int i = 0; i < K; ++i) {
         if (i < kout) {
@@ -451,9 +444,7 @@ __global__ void __launch_bounds__(FB_THREADS)
         QueryRegs q;
         q.set(src[p.q_ox], src[p.q_oy], src[2 * p.q_sc], p.q_xzy != 0);
         const float *ws = p.ws_ref + (size_t)b * ROWS * p.Npad;
-        const int *rperm = p.rperm ? p.rperm + (size_t)b * p.N : nullptr;
-        const size_t orow = p.qperm ? (size_t)b * p.S + p.qperm[qrow] : (size_t)qrow;  // original row
-        auto key_of = [&](int j) {  // j < Npad: packed position; the key carries the original index
+        auto key_of = [&](int j) {  // j < Npad
             const float X = ws[j], Y = ws[p.Npad + j], Z = ws[2 * (size_t)p.Npad + j],
                         W = ws[3 * (size_t)p.Npad + j];
             float d;
@@ -469,7 +460,7 @@ __global__ void __launch_bounds__(FB_THREADS)
                 d = __fmaf_rn(dz, dz, __fmaf_rn(dx, dx, __fmul_rn(dy, dy)));
             }
             if (W == __int_as_float(0x7f800000)) d = W;  // padding
-            return make_key(d, (uint32_t)((rperm && j < p.N) ? rperm[j] : j));
+            return make_key(d, (uint32_t)j);
         };
         int nbest = 0;  // keys carried from the previous segments: list[0 .. nbest)
         for (int seg0 = 0; seg0 < p.Npad; seg0 += FB_SEG) {
@@ -502,11 +493,12 @@ __global__ void __launch_bounds__(FB_THREADS)
         if (tid < kout) {
             const unsigned long long k = list[tid];
             const uint32_t id = (uint32_t)k;
+            const size_t o = (size_t)qrow * kout + tid;
             if (idx_is_int64)
-                reinterpret_cast<long long *>(idx)[orow * kout + tid] = (long long)id;
+                reinterpret_cast<long long *>(idx)[o] = (long long)id;
             else
-                reinterpret_cast<int *>(idx)[orow * kout + tid] = (int)id;
-            if (dist) dist[orow * kout + tid] = sortable2f((uint32_t)(k >> 32));
+                reinterpret_cast<int *>(idx)[o] = (int)id;
+            if (dist) dist[o] = sortable2f((uint32_t)(k >> 32));
         }
         __syncthreads();
     }
@@ -551,7 +543,6 @@ __global__ void knn_merge_kernel(long long nq, int nsplit, int kout,
 struct KnnPlan {
     int Npad, total_tiles, nsplit, tiles_per_split, Kc, qpb;
     int use_est, safe, Spad, R;  // use_est: two-pass path; safe: its bound is guaranteed (k <= 4)
-    int use_tc;                  // two-pass path with the filter on the tensor cores
     int cap;                     // two-pass path: candidate keys per (query, split)
     int tau_tc, SpadT;           // threshold pre-pass on the tensor cores: sample slots (multiple of 1024)
     long long warps;  // warps of the streaming grid (one per 128 queries per split per cloud)
@@ -559,14 +550,10 @@ struct KnnPlan {
     size_t cand_bytes;  // two-pass KNN: candidate lists + counters (shares the pend/state region)
     size_t tc_bytes;    // split-TF32 operand of the refs (tensor-core filter)
     size_t tcs_bytes;   // ... and of the pre-pass sample
-    // spatially sorted clouds (nbr_sort.cuh): sorted copies, permutations, tile boxes
-    int sort;
-    size_t sq_bytes, sr_bytes, qperm_bytes, rperm_bytes, qbox_bytes, rbox_bytes;
-    size_t sort_bytes() const { return sq_bytes + sr_bytes + qperm_bytes + rperm_bytes + qbox_bytes + rbox_bytes; }
     size_t total() const {
         const size_t a = pend_bytes + state_bytes;
         return ws_ref_bytes + samp_bytes + tau_bytes + fail_bytes + part_bytes +
-               (a > cand_bytes ? a : cand_bytes) + tc_bytes + tcs_bytes + sort_bytes();
+               (a > cand_bytes ? a : cand_bytes) + tc_bytes + tcs_bytes;
     }
 };
 
@@ -586,17 +573,9 @@ static bool est_path_pays(int B, int S, int N) {
 }
 static int g_topk_balance = 1;  // key 20 (tests): 0 = thread t of the top-k kernel takes query t
 static int g_topk_split = 1;  // key 18 (tests): 0 = always the thread-per-query top-k kernel
-static int g_tau_tc = 1;  // key 9 (tests): 0 = FP32-pipe threshold pre-pass (knn_tau_kernel)
-// key 17: 1 = Morton-sort the clouds and skip ref tiles whose box cannot hold a candidate
-// (nbr_sort.cuh), 2 = sort without culling. EXPERIMENTAL, off by default: measured on the synthetic
-// LiDAR frames (DESIGN 5.1 "Tried and measured worse") the 128-point tiles of a Morton order span
-// ~12 m boxes against bounds of ~1 m, so a 256-query CTA still keeps 58 % of the tiles, the sort
-// costs 0.2 ms per call, and spatially concentrated candidates overflow the per-split lists.
-static int g_sort = 0;
 // developer: redo counters of the calling thread's last two-pass call (debug_get 5 / 6); every
 // two-pass call writes it, so it is per thread like the library's other state
 static thread_local const int *g_last_fail = nullptr;
-static int g_use_tc = 1;  // key 8 (tests): 0 = FP32-pipe filter (knn_scan_eval_kernel) instead of the tensor-core one
 // key 3: time the dominant kernel of every b200pci_knn call (knn_scan_kernel on the two-pass path,
 // knn_kernel otherwise) with CUDA events on the launching stream; b200pci_debug_get(3) -> accumulated ms, (4) -> number of timed launches.
 static int g_time_kernel = 0;
@@ -627,7 +606,9 @@ static int round_k(int k) {
 // Split the refs of one cloud over several CTAs when the query tiles alone cannot fill the GPU
 // (small B*S), trading a merge pass for occupancy: pick the smallest split count that brings
 // the wave efficiency units / (slots * ceil(units / slots)) above 90 %, if one exists.
-static KnnPlan make_plan(int B, int S, int N, int k, int rows, bool allow_split, bool allow_tc = true) {
+// tc_split = false: the split rule of ball query's scan (knn_scan_kernel, one warp per 128 queries)
+// instead of the tensor-core scan's.
+static KnnPlan make_plan(int B, int S, int N, int k, int rows, bool allow_split, bool tc_split = true) {
     KnnPlan pl;
     pl.total_tiles = ceil_div(N > 0 ? N : 1, NBR_TILE);
     pl.Npad = pl.total_tiles * NBR_TILE;
@@ -642,9 +623,8 @@ static KnnPlan make_plan(int B, int S, int N, int k, int rows, bool allow_split,
                  (pl.safe ? (N >= KNN_SAFE_MIN_N && (long long)B * S * N >= g_safe_min_pairs)
                           : est_path_pays(B, S, N)) &&
                  (long long)B * S < (1LL << 31);
-    pl.use_tc = pl.use_est && g_use_tc && allow_tc;
     int nsplit = 1;
-    if (pl.use_tc) {
+    if (pl.use_est && tc_split) {
         // one CTA per SM, 512 queries per CTA: the split count with the cheapest schedule
         // (waves x (tiles per split + a start-up cost of ~6 tiles))
         const long long tcc = (long long)ceil_div(S, 128 * TC_UNITS) * B;
@@ -691,18 +671,10 @@ static KnnPlan make_plan(int B, int S, int N, int k, int rows, bool allow_split,
     pl.cand_bytes = 0;
     pl.cap = 0;
     // split-TF32 operand [B][Npad][16] followed by the exact |r|^2 row [B][Npad]
-    pl.tc_bytes = pl.use_tc ? align_up((size_t)B * pl.Npad * 17 * sizeof(float), 256) : 0;
-    pl.tau_tc = pl.use_tc && g_tau_tc && ceil_div(N, NBR_SAMPLE_STRIDE) >= 1024;
+    pl.tc_bytes = pl.use_est ? align_up((size_t)B * pl.Npad * 17 * sizeof(float), 256) : 0;
+    pl.tau_tc = pl.use_est && ceil_div(N, NBR_SAMPLE_STRIDE) >= 1024;
     pl.SpadT = pl.tau_tc ? ceil_div(ceil_div(N, NBR_SAMPLE_STRIDE), 1024) * 1024 : 0;
     pl.tcs_bytes = pl.tau_tc ? align_up((size_t)B * pl.SpadT * 16 * sizeof(float), 256) : 0;
-    // Spatial sort + tile culling: tensor-core scan, clouds that fit the sort kernel's shared memory
-    pl.sort = pl.use_tc && g_sort && N <= SORT_MAX_POINTS && S <= SORT_MAX_POINTS && N >= 1 && S >= 1;
-    pl.sq_bytes = pl.sort ? align_up((size_t)B * S * 3 * sizeof(float), 256) : 0;
-    pl.sr_bytes = pl.sort ? align_up((size_t)B * N * 3 * sizeof(float), 256) : 0;
-    pl.qperm_bytes = pl.sort ? align_up((size_t)B * S * sizeof(int), 256) : 0;
-    pl.rperm_bytes = pl.sort ? align_up((size_t)B * N * sizeof(int), 256) : 0;
-    pl.qbox_bytes = pl.sort ? align_up((size_t)B * ceil_div(S, SORT_BLOCK) * 8 * sizeof(float), 256) : 0;
-    pl.rbox_bytes = pl.sort ? align_up((size_t)B * pl.total_tiles * 8 * sizeof(float), 256) : 0;
     if (pl.use_est) {  // the two-pass KNN path needs neither `part` nor `state`
         pl.part_bytes = pl.state_bytes = 0;
         // (an unsplit scan puts all of a query's candidates into one list: twice the room)
@@ -833,30 +805,20 @@ static int launch_topk(const NbrParams &p, int B, const TopkParams &tp, cudaStre
 template <int MODE>
 static int run_two_pass(const KnnPlan &pl, const NbrParams &p, int B, int k, void *idx,
                         int idx_is_int64, float *dist, int *fail_count, int *fail_list,
-                        void *cand_region, const float *ws_tc, TopkParams &tp, cudaStream_t st) {
+                        void *cand_region, TopkParams &tp, cudaStream_t st) {
     ScanEvalParams ep;
     ep.cand = reinterpret_cast<unsigned long long *>(cand_region);
     ep.cand_cnt = reinterpret_cast<uint32_t *>(
         reinterpret_cast<char *>(cand_region) +
         align_up((size_t)pl.warps * pl.cap * 128 * sizeof(unsigned long long), 256));
     ep.cap = pl.cap;
-    dim3 grid(ceil_div(p.S, NBR_QT * 32), p.nsplit, B);
-    if (pl.use_tc) {
-        const bool cull = p.cull != 0 && p.rperm != nullptr && p.tiles_per_split <= 128;
-        auto kern = cull ? knn_scan_tc_kernel<MODE, true> : knn_scan_tc_kernel<MODE, false>;
-        B200PCI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ScanTcSmem::total));
-        dim3 tgrid(ceil_div(p.S, 128 * TC_UNITS), p.nsplit, B);
-        const bool timed = kt_begin(st);  // measurement hook: the scan kernel alone
-        kern<<<tgrid, TC_THREADS, ScanTcSmem::total, st>>>(p, ep, ws_tc);
-        if (timed) kt_end(st);
-        B200PCI_LAUNCH_CHECK("knn_scan_tc_kernel");
-    } else {
-        const size_t smem = ScanEvalSmem<KNN_STAGES>::total;
-        const bool timed = kt_begin(st);  // measurement hook: the scan kernel alone
-        knn_scan_eval_kernel<MODE><<<grid, 32, smem, st>>>(p, ep);
-        if (timed) kt_end(st);
-        B200PCI_LAUNCH_CHECK("knn_scan_eval_kernel");
-    }
+    auto kern = knn_scan_tc_kernel<MODE>;
+    B200PCI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ScanTcSmem::total));
+    dim3 tgrid(ceil_div(p.S, 128 * TC_UNITS), p.nsplit, B);
+    const bool timed = kt_begin(st);  // measurement hook: the scan kernel alone
+    kern<<<tgrid, TC_THREADS, ScanTcSmem::total, st>>>(p, ep);
+    if (timed) kt_end(st);
+    B200PCI_LAUNCH_CHECK("knn_scan_tc_kernel");
     tp.idx = idx;
     tp.dist = dist;
     tp.idx_is_int64 = idx_is_int64;
@@ -865,8 +827,7 @@ static int run_two_pass(const KnnPlan &pl, const NbrParams &p, int B, int k, voi
     tp.fail_list = fail_list;
     tp.cand = ep.cand;
     tp.cand_cnt = ep.cand_cnt;
-    tp.qperm = p.qperm;
-    tp.scan_tiles = (int)grid.x;
+    tp.scan_tiles = ceil_div(p.S, 128);  // 128-query units of a cloud
     tp.nsplit = p.nsplit;
     tp.cap = ep.cap;
     tp.balance = g_topk_balance;
@@ -913,72 +874,24 @@ static SideStream *side_stream() {
 
 // pack -> [tau pre-pass] -> streaming selection -> [merge] -> [exact redo of failed queries]
 template <int MODE>
-static int run_knn(const KnnPlan &pl, const NbrParams &p_in, int B, int k, const float *r,
+static int run_knn(const KnnPlan &pl, const NbrParams &p, int B, int k, const float *r,
                    long long r_sb, long long r_sp, long long r_sc, float *ws_samp, float *tau,
                    void *idx, int idx_is_int64, float *dist, unsigned long long *part,
                    unsigned long long *state, int *fail_count, int *fail_list, float *ws_tc,
-                   char *ws_sort, cudaStream_t st) {
-    NbrParams p = p_in;
+                   cudaStream_t st) {
     const int swap_xy = p.q_ox != 0;
-    // the refs as the pack kernels see them (the sorted copy when the clouds are sorted)
-    const float *rp = r;
-    long long rp_sb = r_sb, rp_sp = r_sp, rp_sc = r_sc;
-    if (pl.sort) {
-        float *sq = reinterpret_cast<float *>(ws_sort);
-        float *sr = reinterpret_cast<float *>(ws_sort + pl.sq_bytes);
-        int *qperm = reinterpret_cast<int *>(ws_sort + pl.sq_bytes + pl.sr_bytes);
-        int *rperm = reinterpret_cast<int *>(ws_sort + pl.sq_bytes + pl.sr_bytes + pl.qperm_bytes);
-        float *qbox = reinterpret_cast<float *>(ws_sort + pl.sq_bytes + pl.sr_bytes + pl.qperm_bytes + pl.rperm_bytes);
-        float *rbox = reinterpret_cast<float *>(ws_sort + pl.sq_bytes + pl.sr_bytes + pl.qperm_bytes + pl.rperm_bytes + pl.qbox_bytes);
-        // a cloud searched against itself (the model's N x N calls) is sorted once
-        const bool same = p.q == r && p.S == p.N && p.q_sb == r_sb && p.q_sp == r_sp && p.q_sc == r_sc;
-        const SortCloud cr = {r, r_sb, r_sp, r_sc, p.N, rperm, sr, rbox};
-        const SortCloud cq = {p.q, p.q_sb, p.q_sp, p.q_sc, p.S, qperm, sq, qbox};
-        int P = 1;
-        while (P < (p.N > p.S ? p.N : p.S)) P <<= 1;
-        const size_t smem = (size_t)P * sizeof(unsigned long long);
-        B200PCI_CUDA(cudaFuncSetAttribute(nbr_sort_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        nbr_sort_kernel<<<dim3(same ? 1 : 2, B), SORT_THREADS, smem, st>>>(cr, cq);
-        B200PCI_LAUNCH_CHECK("nbr_sort_kernel");
-        p.q = same ? sr : sq;
-        p.q_sb = (long long)p.S * 3;
-        p.q_sp = 3;
-        p.q_sc = 1;
-        p.q_ox = swap_xy ? 1 : 0;
-        p.q_oy = swap_xy ? 0 : 1;
-        p.qperm = same ? rperm : qperm;
-        p.rperm = rperm;
-        p.rboxes = rbox;
-        p.cull = 1;
-        rp = sr;
-        rp_sb = (long long)p.N * 3;
-        rp_sp = 3;
-        rp_sc = 1;
-    }
-    if (pl.use_tc) {
+    if (pl.use_est) {
         dim3 grid(ceil_div(pl.Npad, 256), B);
-        // The threshold pre-pass estimates a bound from bucket minima of the 1-in-8 SAMPLE, which
-        // presumes the sample is in no particular spatial order: with sorted clouds it is taken from
-        // the refs as given (a second, sample-only launch), not from the sorted copy.
-        float *tcs = pl.tau_tc ? ws_tc + pl.tc_bytes / sizeof(float) : nullptr;
-        nbr_pack_tc_kernel<<<grid, 256, 0, st>>>(p.N, pl.Npad, rp, rp_sb, rp_sp, rp_sc, swap_xy ? rp_sc : 0,
-                                                 swap_xy ? 0 : rp_sc, ws_tc, pl.sort ? nullptr : tcs, pl.SpadT,
+        nbr_pack_tc_kernel<<<grid, 256, 0, st>>>(p.N, pl.Npad, r, r_sb, r_sp, r_sc, swap_xy ? r_sc : 0,
+                                                 swap_xy ? 0 : r_sc, ws_tc,
+                                                 pl.tau_tc ? ws_tc + pl.tc_bytes / sizeof(float) : nullptr, pl.SpadT,
                                                  ws_tc + (size_t)B * pl.Npad * 16, p.r_xzy);
-        if (pl.sort && tcs != nullptr) {
-            dim3 sgrid(ceil_div(pl.SpadT, 256), B);
-            nbr_pack_tc_kernel<<<sgrid, 256, 0, st>>>(p.N, pl.Npad, r, r_sb, r_sp, r_sc, swap_xy ? r_sc : 0,
-                                                      swap_xy ? 0 : r_sc, nullptr, tcs, pl.SpadT);
-        }
         B200PCI_LAUNCH_CHECK("nbr_pack_tc_kernel");
     }
-    int rc = pack_refs(B, p.N, pl.Npad, rp, rp_sb, rp_sp, rp_sc, const_cast<float *>(p.ws_ref),
+    int rc = pack_refs(B, p.N, pl.Npad, r, r_sb, r_sp, r_sc, const_cast<float *>(p.ws_ref),
                        const_cast<float *>(p.ws_grp), st, pl.Spad,
-                       (pl.use_est && !pl.tau_tc && !pl.sort) ? ws_samp : nullptr, swap_xy, p.r_xzy);
+                       (pl.use_est && !pl.tau_tc) ? ws_samp : nullptr, swap_xy, p.r_xzy);
     if (rc) return rc;
-    if (pl.sort && pl.use_est && !pl.tau_tc) {  // sample rows from the refs as given (see above)
-        rc = pack_refs(B, p.N, pl.Npad, r, r_sb, r_sp, r_sc, nullptr, nullptr, st, pl.Spad, ws_samp, swap_xy, p.r_xzy);
-        if (rc) return rc;
-    }
     if (pl.use_est) {
         g_last_fail = fail_count;
         B200PCI_CUDA(cudaMemsetAsync(fail_count, 0, 256 + (size_t)B * p.S * sizeof(int), st));  // count + flags
@@ -987,7 +900,7 @@ static int run_knn(const KnnPlan &pl, const NbrParams &p_in, int B, int k, const
     }
     TopkParams tp;
     if (pl.use_est) {
-        rc = run_two_pass<MODE>(pl, p, B, k, idx, idx_is_int64, dist, fail_count, fail_list, p.pend, ws_tc, tp, st);
+        rc = run_two_pass<MODE>(pl, p, B, k, idx, idx_is_int64, dist, fail_count, fail_list, p.pend, tp, st);
     } else {
         const bool timed = kt_begin(st);
         rc = dispatch_knn<MODE>(pl.Kc, p, B, idx, idx_is_int64, dist, part, state, k, st);
@@ -1026,8 +939,7 @@ static int run_knn(const KnnPlan &pl, const NbrParams &p_in, int B, int k, const
         int P = MID_MAXP;
         while (P > 1 && p.N / P < 64) P /= 2;
         const size_t smem = (size_t)P * MID_WARP_SMEM;
-        // (the tile-wise redo reads the ORIGINAL refs: its keys are original indices by construction)
-        const MidArgs ma = {p.S, p.N, P, p.q, p.q_sb, p.q_sp, p.q_sc, r, r_sb, r_sp, r_sc, swap_xy, p.q_xzy, p.r_xzy, p.qperm, idx,
+        const MidArgs ma = {p.S, p.N, P, p.q, p.q_sb, p.q_sp, p.q_sc, r, r_sb, r_sp, r_sc, swap_xy, p.q_xzy, p.r_xzy, idx,
                             idx_is_int64, dist, k, fail_list, fail_list + (size_t)B * p.S, fail_count};
         if (pl.Kc <= 16) {
             auto kern = knn_redo_kernel<MODE, 16>;
@@ -1082,7 +994,7 @@ static int knn_impl(int B, int S, int N, int k, int mode, const float *q, long l
         while (P < 8 && qwarps * P < 8LL * sm_count() && N / (2 * P) >= 64) P *= 2;
         const size_t smem = (size_t)P * MID_WARP_SMEM;
         dim3 grid(ceil_div(S, 32), B);
-        const MidArgs ma = {S, N, P, q, q_sb, q_sp, q_sc, r, r_sb, r_sp, r_sc, swap_xy, q_xzy, r_xzy, nullptr, idx,
+        const MidArgs ma = {S, N, P, q, q_sb, q_sp, q_sc, r, r_sb, r_sp, r_sc, swap_xy, q_xzy, r_xzy, idx,
                             idx_is_int64, dist, k, nullptr, nullptr, nullptr};
 #define B200PCI_MID(MM, KK)                                                                       \
     do {                                                                                          \
@@ -1131,7 +1043,6 @@ static int knn_impl(int B, int S, int N, int k, int mode, const float *q, long l
     if (!pl.use_est) fail_count = fail_list = nullptr;
     const size_t shared_region = pl.pend_bytes + pl.state_bytes > pl.cand_bytes ? pl.pend_bytes + pl.state_bytes : pl.cand_bytes;
     float *ws_tc = reinterpret_cast<float *>(wsp + pl.part_bytes + shared_region);
-    char *ws_sort = wsp + pl.part_bytes + shared_region + pl.tc_bytes + pl.tcs_bytes;
 
     NbrParams p;
     p.S = S;
@@ -1148,11 +1059,9 @@ static int knn_impl(int B, int S, int N, int k, int mode, const float *q, long l
     p.q_oy = swap_xy ? 0 : q_sc;
     p.q_xzy = q_xzy;
     p.r_xzy = r_xzy;
-    p.rperm = p.qperm = nullptr;
-    p.rboxes = nullptr;
-    p.cull = 0;
     p.ws_ref = ws_ref;
     p.ws_grp = ws_ref + (size_t)B * 4 * pl.Npad;
+    p.ws_tc = ws_tc;
     p.tau_in = pl.use_est ? tau : nullptr;
     p.pend = pend;
     p.pend_cnt = pend + (size_t)pl.warps * NBR_QT * (SCAN_CAP > NBR_CAP ? SCAN_CAP : NBR_CAP) * 32;
@@ -1160,10 +1069,10 @@ static int knn_impl(int B, int S, int N, int k, int mode, const float *q, long l
     int rc = (mode == B200PCI_DIST_EXPANDED)
                  ? run_knn<B200PCI_DIST_EXPANDED>(pl, p, B, k, r, r_sb, r_sp, r_sc, ws_samp, tau, idx,
                                                   idx_is_int64, dist, part, state, fail_count,
-                                                  fail_list, ws_tc, ws_sort, st)
+                                                  fail_list, ws_tc, st)
                  : run_knn<B200PCI_DIST_DIRECT>(pl, p, B, k, r, r_sb, r_sp, r_sc, ws_samp, tau, idx,
                                                 idx_is_int64, dist, part, state, fail_count,
-                                                fail_list, ws_tc, ws_sort, st);
+                                                fail_list, ws_tc, st);
     return rc;
 }
 
@@ -1533,11 +1442,9 @@ extern "C" int b200pci_ball_query(int b, int n, int m, float radius, int nsample
     p.q_ox = 0;
     p.q_oy = 1;
     p.q_xzy = p.r_xzy = 0;
-    p.rperm = p.qperm = nullptr;
-    p.rboxes = nullptr;
-    p.cull = 0;
     p.ws_ref = ws_ref;
     p.ws_grp = ws_ref + (size_t)b * 4 * pl.Npad;
+    p.ws_tc = nullptr;
     p.tau_in = nullptr;
     p.tau_uniform = radius * radius;  // FP32, ball_query_gpu.cu:24
     p.pend = reinterpret_cast<uint32_t *>(wsb + pl.ws_ref_bytes);
@@ -1645,11 +1552,11 @@ extern "C" int b200pci_knn_backward(int B, int S, int N, int K, const float *q, 
     return B200PCI_OK;
 }
 
-// Test hooks: key 1 = scale applied to the estimated admission bound (1.0 = production),
-// key 2 = 1 disables the estimate (exact streaming only), key 6 = 1 sends every ball query through
-// the exact redo kernel, key 7 = pair count from which k <= 4 takes the two-pass path (0 = default),
-// key 3 = 1 starts (and resets) CUDA-event
-// timing of the selection kernel. Process-global, not thread-safe.
+// Test hooks (every key is listed in include/b200pci.h): key 1 = scale applied to the estimated
+// admission bound (1.0 = production), key 2 = 1 disables the estimate (exact streaming only), key 6 =
+// 1 sends every ball query through the exact redo kernel, key 7 = pair count from which k <= 4 takes
+// the two-pass path (0 = default), key 3 = 1 starts (and resets) CUDA-event timing of the selection
+// kernel. A key not listed there returns B200PCI_EINVAL. Process-global, not thread-safe.
 extern "C" int b200pci_debug_set(int key, double value) {
     if (key == 1)
         g_tau_scale = (float)value;
@@ -1664,18 +1571,12 @@ extern "C" int b200pci_debug_set(int key, double value) {
         g_ball_force_redo = value != 0.0;
     else if (key == 7)
         g_safe_min_pairs = value > 0.0 ? (long long)value : KNN_SAFE_MIN_PAIRS;
-    else if (key == 8)
-        g_use_tc = value != 0.0;
-    else if (key == 9)
-        g_tau_tc = value != 0.0;
     else if (key == 12)
         g_est_min_n = value > 0.0 ? (int)value : 2048;
     else if (key == 13)
         g_est_min_pairs = value > 0.0 ? (long long)value : (1LL << 25);
     else if (key == 11)
         g_R_override = (int)value;
-    else if (key == 17)
-        g_sort = (int)value;
     else if (key == 18)
         g_topk_split = (int)value;
     else if (key == 20)

@@ -10,8 +10,8 @@
 //     (sortable(distance) << 32 | index: the lowest index wins ties) held in registers;
 //   * nbr_stream + TopKSink: the single-kernel engine (scan + pending lists in global memory +
 //     drains + sorting-network folds) that serves k = 33..64 and the exact mode of the test hooks.
-//     The big cases run on nbr_scan_eval.cuh (scan + evaluate, then top-k), ball_query on
-//     nbr_two_pass.cuh, the small ones on knn_mid_kernel (knn.cu).
+//     The big cases run on nbr_scan_tc.cuh (scan + evaluate) and nbr_topk.cuh (top-k), ball_query
+//     on nbr_two_pass.cuh, the small ones on knn_mid_kernel (knn.cu).
 //
 // In-kernel engine: a warp owns QT*32 queries (4 per thread, in registers) of one cloud and one
 // split of the refs. It streams the 128-ref tiles of the SoA rows through its OWN small
@@ -33,6 +33,10 @@ constexpr int NBR_BLK = 8;         // groups per scan step
 constexpr int NBR_CAP = 64;        // pending entries per query slot (global memory)
 constexpr int NBR_SAMPLE_STRIDE = 8;  // the threshold pre-pass looks at every 8th ref
 
+// Passed by value to the search kernels. Its size is above 128 bytes, and that matters: nvcc
+// lowers the reads of a by-value kernel argument of at most 128 bytes differently, which
+// reschedules every kernel that takes one (knn_scan_tc_kernel<0>, issue-bound: 1392 instead of
+// 1368 SASS instructions when this struct was 128 bytes).
 struct NbrParams {
     int S, N, Npad;
     int nsplit, tiles_per_split, total_tiles;
@@ -44,16 +48,14 @@ struct NbrParams {
     const float *ws_ref;  // [B][4][Npad] rows (streamed by the scan)
     const float *ws_grp;  // [B][Npad/4][4][4] the same refs, one 64-byte record per group of 4
                           // (x[4] y[4] z[4] w[4]): what a drain gathers, 2 sectors per group
-    // spatially sorted clouds (nbr_sort.cuh; null / 0 when the call runs on the clouds as given):
-    const int *rperm;      // [B][N] packed ref position -> original ref index (what the keys carry)
-    const int *qperm;      // [B][S] query row processed here -> original query row (where results go)
-    const float *rboxes;   // [B][total_tiles][8] bounding boxes of the 128-ref tiles
-    int cull;              // tensor-core scan: skip ref tiles that cannot hold a candidate
+    const float *ws_tc;   // tensor-core scan: [B][Npad][16] split-TF32 operand, then the exact |r|^2
+                          // rows [B][Npad] (nbr_pack_tc_kernel)
     const float *tau_in;  // two-pass scans: [B][S] admission bounds (null: tau_uniform for every query)
     float tau_uniform;
     uint32_t *pend;       // [warps][QT][CAP/4][32][4] pending entries
     uint32_t *pend_cnt;   // two-pass path: [warps][QT][32] list lengths
 };
+static_assert(sizeof(NbrParams) > 128, "NbrParams: see the size note above");
 
 // ---- pack kernel ---------------------------------------------------------------------------
 // Packed reference rows (both distance forms): x, y, z and the FILTER addend

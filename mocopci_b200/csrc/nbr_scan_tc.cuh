@@ -15,8 +15,7 @@
 // stays CONSERVATIVE through a 2^-16 relative slack on |r|^2 (inside w') and on |q|^2 (inside
 // thr), 14x that bound: no pair below the admission bound is ever missed, candidate <=> D < 0. The
 // flagged groups are re-evaluated in the exact reference arithmetic (FP32 pipe, dist4 of
-// nbr_engine.cuh); the top-k kernel is unchanged. Results are bit-identical to the FP32-pipe
-// generation (nbr_scan_eval.cuh), which test hook 8 = 0 still selects.
+// nbr_engine.cuh) and the candidates go to the lists that the top-k kernels of nbr_topk.cuh read.
 //
 // Operand layout: K-major, no swizzle. A tile of 128 rows is [k/4][row][4 floats]: 8 rows x 16 B
 // form one 128-byte core matrix, SBO = 128 B between 8-row groups, LBO = 2048 B between the four
@@ -38,8 +37,7 @@
 //                while waiting for an accumulator.
 // knn_tau_tc_kernel: the threshold pre-pass on the same pipeline over the packed 1-in-8 sample.
 #pragma once
-#include "nbr_scan_eval.cuh"
-#include "nbr_sort.cuh"
+#include "nbr_topk.cuh"
 
 namespace b200pci {
 
@@ -91,7 +89,7 @@ struct ScanTcSmem {
     static constexpr size_t qtab = (size_t)TC_UNITS * 5 * 128 * sizeof(float);
     static constexpr size_t queue = (size_t)TC_EPI_WARPS * 2 * TC_QCAP * sizeof(uint32_t);
     static constexpr size_t cnt = (size_t)TC_UNITS * 128 * sizeof(uint32_t);
-    static constexpr size_t ctrl = 2048;  // mbarriers (1152 B), TMEM slot, query box, kept-tile list
+    static constexpr size_t ctrl = 2048;  // mbarriers (1152 B), TMEM slot
     static constexpr size_t used = ring + aop + qtab + queue + cnt + ctrl;
     // two units: more than half of the SM's shared memory, one CTA per SM (it allocates all of TMEM)
     static constexpr size_t total = (TC_UNITS == 1 || used > 120 * 1024) ? used : 120 * 1024;
@@ -261,13 +259,10 @@ __device__ __forceinline__ uint32_t tc_step_mask(const float (&v)[32]) {
 // flagged groups go back to the head of the queue for the next round.
 // Runs rounds while at least 32 items are queued, or the oldest item is from a tile before
 // `min_tile` (the tile has to leave the ring). Returns the tile of the oldest item left.
-// CULL: the experimental sorted / culled variant (nbr_sort.cuh); the default instantiation carries
-// none of its code (the scan is issue-bound: the extra address selects alone cost 8 %).
-template <int MODE, bool CULL>
+template <int MODE>
 __device__ __noinline__ int tc_drain(uint32_t *qm, uint32_t *qi, uint32_t &qhead, uint32_t qtail, int min_tile, int max_rounds,
                                      const float *qt, int quarter, int half, const unsigned char *ring, int t_now,
-                                     int tile0, int N, uint32_t *ccnt, u64 *cand_unit, uint32_t cap,
-                                     const uint16_t *klist, const int *rperm) {
+                                     int tile0, int N, uint32_t *ccnt, u64 *cand_unit, uint32_t cap) {
     constexpr int G4 = NBR_TILE / 4;
     const int lane = threadIdx.x & 31;
     const uint32_t lt_mask = (1u << lane) - 1u;
@@ -301,16 +296,13 @@ __device__ __noinline__ int tc_drain(uint32_t *qm, uint32_t *qi, uint32_t &qhead
         const float4 X = sX[g], Y = sX[G4 + g], Z = sX[2 * G4 + g];
         const float4 Wn = mode_expanded(MODE) ? sX[3 * G4 + g] : make_float4(0.f, 0.f, 0.f, 0.f);
         float d[4];
-        // `tile` counts the tiles this CTA streams; with culling that is a position in its kept list
-        const uint32_t i0 = ((uint32_t)(tile0 + (CULL ? (int)klist[e ? tile : 0] : tile)) * G4 + g) * 4u;
+        const uint32_t i0 = ((uint32_t)(tile0 + tile) * G4 + g) * 4u;
         dist4n<MODE>(q, X, Y, Z, Wn, i0, N, d);
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
             if (e && d[i] < tau) {
                 const uint32_t slot = atomicAdd(&ccnt[owner], 1u);
-                // sorted clouds: the key carries the ORIGINAL ref index (ties -> lowest original index)
-                if (slot < cap)
-                    cand_unit[(size_t)slot * 128 + owner] = make_key(d[i], CULL ? (uint32_t)__ldg(rperm + i0 + i) : i0 + i);
+                if (slot < cap) cand_unit[(size_t)slot * 128 + owner] = make_key(d[i], i0 + i);
             }
         }
         const bool left = m != 0u;
@@ -328,8 +320,8 @@ __device__ __noinline__ int tc_drain(uint32_t *qm, uint32_t *qi, uint32_t &qhead
     return oldest;
 }
 
-template <int MODE, bool CULL>
-__device__ __forceinline__ void nbr_scan_tc(const NbrParams &p, const ScanEvalParams &ep, const float *ws_tc) {
+template <int MODE>
+__device__ __forceinline__ void nbr_scan_tc(const NbrParams &p, const ScanEvalParams &ep) {
     using SM = ScanTcSmem;
     constexpr int G4 = NBR_TILE / 4;
     extern __shared__ __align__(128) unsigned char smem[];
@@ -344,30 +336,14 @@ __device__ __forceinline__ void nbr_scan_tc(const NbrParams &p, const ScanEvalPa
     uint64_t *bfull = bars + 2 * TC_STAGES, *bempty = bfull + TC_BSTAGES;  // operand ring
     uint64_t *acc_full = bempty + TC_BSTAGES, *acc_empty = acc_full + 2 * TC_UNITS;  // [unit][buffer]
     uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(acc_empty + 2 * TC_UNITS);
-    // culling (sorted clouds): the CTA's query box as order-preserving integers [lo.xyz, hi.xyz,
-    // max tau, max |q|^2], the number of kept tiles and their list
-    uint32_t *qbox = tmem_slot + 2;
-    int *nkept = reinterpret_cast<int *>(qbox + 8);
-    uint16_t *klist = reinterpret_cast<uint16_t *>(nkept + 2);  // [<= 128]
     unsigned char *sring = ring + ScanTcSmem::bring;
 
     const int b = blockIdx.z, split = blockIdx.y;
     const int tile0 = split * p.tiles_per_split;
-    const int ntiles_all = min(p.tiles_per_split, p.total_tiles - tile0);
-    constexpr bool cull = CULL;  // (the host only picks this instantiation when ntiles_all <= 128)
-    const uint16_t *kl = CULL ? klist : nullptr;
-    const int *rperm = CULL ? p.rperm + (size_t)b * p.N : nullptr;
+    const int ntiles = min(p.tiles_per_split, p.total_tiles - tile0);
     const int scan_units = (p.S + 127) / 128;  // 128-query units of a cloud (= top-k kernel's grid)
 
     if (tid == 0) {
-        if (CULL) {
-            for (int k = 0; k < 3; ++k) {
-                qbox[k] = 0xFFFFFFFFu;  // running minima
-                qbox[3 + k] = 0u;       // running maxima
-            }
-            qbox[6] = qbox[7] = 0u;
-        }
-        if (CULL) *nkept = ntiles_all;
         for (int s = 0; s < TC_STAGES; ++s) {
             mbar_init(&full[s], 1);
             mbar_init(&empty[s], TC_EPI_WARPS);
@@ -389,7 +365,6 @@ __device__ __forceinline__ void nbr_scan_tc(const NbrParams &p, const ScanEvalPa
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
 
-    if (cull) __syncthreads();  // the query box is initialised (uniform over the CTA)
     // epilogue threads: query constants, A operand row, per-query tables
     const int unit = warp >> 3, half = (warp >> 2) & 1, quarter = warp & 3;
     const int owner = quarter * 32 + lane;  // row inside the unit = TMEM lane
@@ -408,26 +383,6 @@ __device__ __forceinline__ void nbr_scan_tc(const NbrParams &p, const ScanEvalPa
         q.set(x, y, z, p.q_xzy != 0);
         const float d0 = __fsub_rn(t0, q.s);
         thr = d0 + (0x1p-16f * q.s + 0x1p-21f * fabsf(d0));
-        if (cull && half == 0) {
-            // box of the CTA's valid queries (original coordinate order: x and y were exchanged
-            // on the way in for DIST_DIRECT_XYZ), their largest bound and largest |q|^2
-            const bool v = qi < p.S;
-            const float inf = __int_as_float(0x7f800000);
-            const float c3[3] = {p.q_ox != 0 ? y : x, p.q_ox != 0 ? x : y, z};
-#pragma unroll
-            for (int k = 0; k < 3; ++k) {
-                const float lo = warp_min_f(v ? c3[k] : inf), hi = warp_max_f(v ? c3[k] : -inf);
-                if (lane == 0) {
-                    atomicMin(&qbox[k], f2sortable(lo));
-                    atomicMax(&qbox[3 + k], f2sortable(hi));
-                }
-            }
-            const float tmax = warp_max_f(v ? t0 : -inf), smax = warp_max_f(v ? q.s : 0.f);
-            if (lane == 0) {
-                atomicMax(&qbox[6], f2sortable(tmax));
-                atomicMax(&qbox[7], f2sortable(smax));
-            }
-        }
         if (half == 0) {  // (both column halves hold the same queries)
         float *qt = qtab_all + unit * (5 * 128);
         qt[owner] = q.fa;
@@ -461,51 +416,21 @@ __device__ __forceinline__ void nbr_scan_tc(const NbrParams &p, const ScanEvalPa
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    if (cull) {
-        // Kept-tile list (producer warp, all lanes): a ref tile whose box is farther from the query
-        // box than the largest bound of the CTA's queries cannot hold a candidate of any of them:
-        // every pair has D_exact >= gap^2 - 2^-20 (|q|^2 + |r|^2) (DESIGN 5.1), and candidates need
-        // D_exact < tau. The slack below is 4x that bound plus the rounding of the gap itself.
-        if (warp == TC_EPI_WARPS) {
-            float qb[6];
-#pragma unroll
-            for (int k = 0; k < 6; ++k) qb[k] = sortable2f(qbox[k]);
-            const float tmax = sortable2f(qbox[6]), smax = sortable2f(qbox[7]);
-            const float *rb0 = p.rboxes + ((size_t)b * p.total_tiles + tile0) * 8;
-            int cnt = 0;
-            for (int t0 = 0; t0 < ntiles_all; t0 += 32) {
-                const int t = t0 + lane;
-                bool keep = false;
-                if (t < ntiles_all) {
-                    const float *rb = rb0 + (size_t)t * 8;
-                    const float gap = box_gap2(qb, rb);
-                    const float slack = 0x1p-18f * (smax + rb[6] + gap);
-                    keep = !(gap - slack >= tmax);  // (NaN anywhere keeps the tile)
-                }
-                const unsigned bal = __ballot_sync(0xffffffffu, keep);
-                if (keep) klist[cnt + __popc(bal & ((1u << lane) - 1u))] = (uint16_t)t;
-                cnt += __popc(bal);
-            }
-            if (lane == 0) *nkept = cnt;
-        }
-        __syncthreads();
-    }
-    const int ntiles = CULL ? *nkept : ntiles_all;
 
     if (warp == TC_EPI_WARPS) {
         // ---- TMA producer ----
         if (lane == 0) {
-            const float *tc_cloud = ws_tc + (size_t)b * p.Npad * 16;
+            const float *tc_cloud = p.ws_tc + (size_t)b * p.Npad * 16;
             const float *ws = p.ws_ref + (size_t)b * 4 * p.Npad;
             // exact |r|^2 row (behind the operands of all clouds): only the expanded forms read it
-            const float *nrm = ws_tc + (size_t)gridDim.z * p.Npad * 16 + (size_t)b * p.Npad;
+            const float *nrm = p.ws_tc + (size_t)gridDim.z * p.Npad * 16 + (size_t)b * p.Npad;
             constexpr uint32_t soa_tx = (mode_expanded(MODE) ? 4u : 3u) * NBR_TILE * sizeof(float);
             for (int t = 0; t < ntiles; ++t) {
                 const int s = t & (TC_STAGES - 1), sb = t & (TC_BSTAGES - 1);
                 const int pp = t >> 1, ps = pp & (TC_STAGES / 2 - 1);  // the SoA barriers count tile PAIRS
                 if (t >= TC_BSTAGES) mbar_wait_suspend(&bempty[sb], ((t / TC_BSTAGES) - 1) & 1);
                 mbar_arrive_expect_tx(&bfull[sb], TC_B_BYTES);
-                const int ta = tile0 + (CULL ? (int)kl[t] : t);  // absolute tile
+                const int ta = tile0 + t;  // absolute tile
                 tma_load_1d(ring + (size_t)sb * TC_B_BYTES, tc_cloud + (size_t)ta * NBR_TILE * 16, TC_B_BYTES, &bfull[sb]);
                 unsigned char *st = sring + (size_t)s * TC_SOA_BYTES;
                 if ((t & 1) == 0) {
@@ -576,8 +501,8 @@ __device__ __forceinline__ void nbr_scan_tc(const NbrParams &p, const ScanEvalPa
                     while (!ready) {
                         ready = __all_sync(0xffffffffu, mbar_try_wait(&acc_full[2 * unit + buf], pr & 1));
                         if (!ready && qtail - qhead >= 32u)
-                            t_oldest = tc_drain<MODE, CULL>(qm, qi, qhead, qtail, -0x40000000, 1, qt, quarter, half, sring, pr, tile0,
-                                                      p.N | (p.r_xzy ? NBR_N_XZY : 0), ccnt, cand_unit, (uint32_t)ep.cap, kl, rperm);
+                            t_oldest = tc_drain<MODE>(qm, qi, qhead, qtail, -0x40000000, 1, qt, quarter, half, sring, pr, tile0,
+                                                      p.N | (p.r_xzy ? NBR_N_XZY : 0), ccnt, cand_unit, (uint32_t)ep.cap);
                     }
 #else
                     mbar_wait(&acc_full[2 * unit + buf], pr & 1);
@@ -615,8 +540,8 @@ __device__ __forceinline__ void nbr_scan_tc(const NbrParams &p, const ScanEvalPa
             const uint32_t size = qtail - qhead;
             const bool last = pr == npairs - 1;
             if (size >= TC_DRAIN_AT_V || (size > 0u && (pr - t_oldest >= TC_HOLD_PAIRS || last)))
-                t_oldest = tc_drain<MODE, CULL>(qm, qi, qhead, qtail, last ? pr + 1 : pr - TC_HOLD_PAIRS + 1, last ? (1 << 30) : TC_ROUNDS_V, qt,
-                                          quarter, half, sring, pr, tile0, p.N | (p.r_xzy ? NBR_N_XZY : 0), ccnt, cand_unit, (uint32_t)ep.cap, kl, rperm);
+                t_oldest = tc_drain<MODE>(qm, qi, qhead, qtail, last ? pr + 1 : pr - TC_HOLD_PAIRS + 1, last ? (1 << 30) : TC_ROUNDS_V, qt,
+                                          quarter, half, sring, pr, tile0, p.N | (p.r_xzy ? NBR_N_XZY : 0), ccnt, cand_unit, (uint32_t)ep.cap);
             const int p_free = (qhead != qtail) ? t_oldest : pr + 1;  // pairs < p_free leave the ring
             __syncwarp();
             if (lane == 0) {

@@ -1,5 +1,5 @@
 // The pending-list flavour of the two-pass path, used by ball_query (DESIGN.md "Neighbourhood
-// searches"; KNN / three_nn / Chamfer use the scan + evaluate kernel of nbr_scan_eval.cuh):
+// searches"; KNN / three_nn / Chamfer use the scan + evaluate kernel of nbr_scan_tc.cuh):
 //
 //   scan   (nbr_scan)          the streaming filter with nothing else in the kernel: a warp owns
 //                              4 x 32 queries and one split of the refs, and appends one

@@ -101,7 +101,7 @@ def knn8_oracle(orc, pairs8):
 def assert_two_pass_knn(names, k, split_topk=False):
     """The two-pass neighbour search: tensor-core scan in the expanded arithmetic, then the top-k
     kernel -- one thread per query, or one thread per (query, group of ref splits)."""
-    assert "knn_scan_tc_kernel<0, false>" in names, names
+    assert "knn_scan_tc_kernel<0>" in names, names
     want = f"knn_topk_split_kernel<{k}>" if split_topk else f"knn_topk_kernel<{k}>"
     other = f"knn_topk_kernel<{k}>" if split_topk else f"knn_topk_split_kernel<{k}>"
     assert want in names and other not in names, names
@@ -304,7 +304,7 @@ def test_chamfer_per_point_vs_oracle(orc, case):
     if case == "uniform_B2":  # the one-launch kernel, both directions
         assert names.count("knn_mid_kernel<1, 16>") == 2 and "knn_scan_tc_kernel" not in base(names), names
     else:  # two-pass search in the direct-difference arithmetic, both directions
-        assert names.count("knn_scan_tc_kernel<1, false>") == 2, names
+        assert names.count("knn_scan_tc_kernel<1>") == 2, names
         assert names.count("knn_topk_kernel<1>") == 2, names
 
 
@@ -467,7 +467,7 @@ def test_three_nn_weights_pyramid_vs_oracle(orc, pairs8):
         np.testing.assert_array_equal(bits(w), bits(ow), err_msg=f"{m}->{n}")
         assert names.count("three_nn_finish_kernel") == 1, (n, m, names)
         if n == NPTS:  # two-pass search in the direct-difference arithmetic
-            assert "knn_scan_tc_kernel<1, false>" in names and "knn_topk_kernel<3>" in names, names
+            assert "knn_scan_tc_kernel<1>" in names and "knn_topk_kernel<3>" in names, names
         else:          # the one-launch kernel
             assert sorted(names) == ["knn_mid_kernel<1, 16>", "three_nn_finish_kernel"], (n, m, names)
 

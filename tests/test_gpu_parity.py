@@ -133,25 +133,22 @@ def test_knn_uniform_vs_oracle(ops, orc, B, S, N, k):
     check_knn_against_oracle(ops, orc, xyz, new, k)
 
 
-@pytest.mark.parametrize("tc", [1, 0])
 @pytest.mark.parametrize("B,S,N,k", [(1, 700, 5000, 1), (2, 300, 3000, 4), (1, 1030, 9000, 3),
                                       (1, 100, 20000, 2)])
-def test_knn_small_k_two_pass_forced(ops, orc, B, S, N, k, tc):
+def test_knn_small_k_two_pass_forced(ops, orc, B, S, N, k):
     """k <= 4 takes the two-pass path (guaranteed sample bound) only from 2^25 pairs; test hook 7
-    lowers that threshold so the oracle can check it on small inputs -- with the tensor-core
-    filter (default) and the FP32-pipe one (hook 8 = 0), EXPANDED (knn_point) and DIRECT (three_nn)."""
+    lowers that threshold so the oracle can check it on small inputs, EXPANDED (knn_point) and
+    DIRECT (three_nn)."""
     from mocopci_b200 import _lib
     xyz = ops.synth.uniform_cloud(300 + N, B, N, -30.0, 30.0).numpy()
     new = ops.synth.uniform_cloud(400 + S, B, S, -30.0, 30.0).numpy()
     try:
-        _lib.check(_lib.lib.b200pci_debug_set(8, tc))
         _lib.check(_lib.lib.b200pci_debug_set(7, 1))
         check_knn_against_oracle(ops, orc, xyz, new, k)
         u, kn = dev(new), dev(xyz)
         dist, idx = ops.p2u.three_nn(u, kn)
     finally:
         _lib.check(_lib.lib.b200pci_debug_set(7, 0))
-        _lib.check(_lib.lib.b200pci_debug_set(8, 1))
     od2, oi = orc.three_nn(new, xyz)
     np.testing.assert_array_equal(idx.cpu().numpy(), oi)
     np.testing.assert_array_equal(bits(dist.cpu().numpy()), bits(np.sqrt(od2)))
@@ -208,22 +205,39 @@ def test_knn_degenerate_cloud_mass_redo(ops, orc):
     check_knn_against_oracle(ops, orc, xyz2, new, 32)
 
 
-@pytest.mark.parametrize("tc", [1, 0])
 @pytest.mark.parametrize("B,S,N,k,lo,hi", [(1, 700, 9000, 16, -1.0, 1.0), (2, 1100, 8192, 32, -50.0, 50.0),
                                             (1, 513, 16500, 8, -80.0, 80.0), (3, 129, 10000, 16, 900.0, 1000.0)])
-def test_knn_two_pass_both_filters_vs_oracle(ops, orc, tc, B, S, N, k, lo, hi):
-    """The two-pass path with the tensor-core filter (tcgen05 TF32, split operands; default) and with
-    the FP32-pipe filter (test hook 8 = 0): both are conservative pre-filters in front of the same
-    exact evaluation, so both must reproduce the oracle bit for bit -- also far from the origin,
-    where the relative slack of the filters is largest in absolute terms."""
-    from mocopci_b200 import _lib
+def test_knn_two_pass_vs_oracle(ops, orc, B, S, N, k, lo, hi):
+    """The two-pass path: the tensor-core filter (tcgen05 TF32, split operands) is a conservative
+    pre-filter in front of the exact evaluation, so the result must reproduce the oracle bit for
+    bit -- also far from the origin, where the relative slack of the filter is largest in absolute
+    terms."""
     xyz = ops.synth.uniform_cloud(700 + N, B, N, lo, hi).numpy()
     new = ops.synth.uniform_cloud(800 + S, B, S, lo, hi).numpy()
-    try:
-        _lib.check(_lib.lib.b200pci_debug_set(8, tc))
-        check_knn_against_oracle(ops, orc, xyz, new, k)
-    finally:
-        _lib.check(_lib.lib.b200pci_debug_set(8, 1))
+    check_knn_against_oracle(ops, orc, xyz, new, k)
+
+
+@pytest.mark.parametrize("k", [1, 3, 16, 32])
+def test_knn_two_pass_clusters_vs_oracle(ops, orc, k):
+    """The two-pass path on two far-apart Gaussian clusters (about +40 m and -55 m) with 1000 exact
+    duplicates, queried by a permuted subset of the cloud: candidates crowd into few ref tiles and
+    tie exactly. Oracle bit for bit in all three arithmetics; hook 7 sends k <= 4 to the two-pass
+    path as well."""
+    from mocopci_b200 import _lib, pointconv_util as pcu
+    g = torch.Generator().manual_seed(k)
+    clusters = torch.cat([torch.randn(2, 9000, 3, generator=g) * 0.5 + 40.0,
+                          torch.randn(2, 7384, 3, generator=g) * 2.0 - 55.0], 1)
+    clusters[:, 100:1100] = clusters[:, 3000:4000]                     # 1000 exact duplicates
+    new = clusters[:, torch.randperm(16384, generator=g)][:, :5000].contiguous()
+    for mode, form in ((pcu.DIST_EXPANDED_CUDA, 5), (pcu.DIST_DIRECT, 1), (pcu.DIST_DIRECT_XYZ, 2)):
+        try:
+            _lib.check(_lib.lib.b200pci_debug_set(7, 1))
+            idx, dist = pcu._knn(k, clusters.cuda(), new.cuda(), mode, True)
+        finally:
+            _lib.check(_lib.lib.b200pci_debug_set(7, 0))
+        oi, od = orc.knn_form(form, k, clusters.numpy(), new.numpy())
+        np.testing.assert_array_equal(idx.cpu().numpy(), oi, err_msg=f"mode {mode}")
+        np.testing.assert_array_equal(bits(dist.cpu().numpy()), bits(od), err_msg=f"mode {mode}")
 
 
 @pytest.mark.parametrize("grid", [6, 20])
@@ -236,23 +250,6 @@ def test_knn_two_pass_tie_stress_vs_oracle(ops, orc, grid):
     for k in (8, 16, 32):
         check_knn_against_oracle(ops, orc, xyz, new, k)
     check_knn_against_oracle(ops, orc, xyz, xyz[:, :1500], 16)  # queries that coincide with refs
-
-
-def test_knn_filters_agree_at_full_size(ops):
-    """BASELINE size (8 x 16384 x 16384, k = 16 and 32, LiDAR frames): tensor-core and FP32-pipe
-    filters give identical indices and distances."""
-    from mocopci_b200 import _lib
-    a, b = ops.synth.frame_pairs(21, 8)
-    a, b = a.cuda(), b.cuda()
-    for k in (16, 32):
-        i1, d1 = ops.pcu.knn_point_with_dist(k, a, b)
-        try:
-            _lib.check(_lib.lib.b200pci_debug_set(8, 0))
-            i0, d0 = ops.pcu.knn_point_with_dist(k, a, b)
-        finally:
-            _lib.check(_lib.lib.b200pci_debug_set(8, 1))
-        assert torch.equal(i1, i0)
-        assert torch.equal(d1.view(torch.int32), d0.view(torch.int32))
 
 
 @pytest.mark.parametrize("k", [3, 16, 32])
@@ -303,44 +300,6 @@ def test_knn_split_topk_kernel_equals_thread_per_query_kernel(ops, k):
             assert torch.equal(i1, i0), f"{name} mode {mode}: {int((i1 != i0).sum())} indices differ"
             assert torch.equal(d1.view(torch.int32), d0.view(torch.int32)), f"{name} mode {mode}"
             assert torch.equal(j1.long(), i0)
-
-
-@pytest.mark.parametrize("k", [1, 3, 16, 32])
-def test_knn_sorted_culled_path_equals_plain_path(ops, orc, k):
-    """Experimental path (test hook 17 = 1, off by default): clouds of up to 16384 points are
-    Morton-sorted and the tensor-core scan skips ref tiles whose box cannot hold a candidate.
-    Results must be IDENTICAL to the plain path --
-    indices (ties by ORIGINAL index), distance bits, row order -- on LiDAR frames, on far-apart
-    clusters with duplicated points, for a cloud searched against itself (sorted once) and for
-    permuted views."""
-    from mocopci_b200 import _lib, pointconv_util as pcu
-    a, b = ops.synth.frame_pairs(60 + k, 2)
-    g = torch.Generator().manual_seed(k)
-    clusters = torch.cat([torch.randn(2, 9000, 3, generator=g) * 0.5 + 40.0,
-                          torch.randn(2, 7384, 3, generator=g) * 2.0 - 55.0], 1)
-    clusters[:, 100:1100] = clusters[:, 3000:4000]                     # 1000 exact duplicates
-    cases = [("lidar", a.cuda(), b.cuda()), ("self", a.cuda(), a.cuda()),
-             ("clusters", clusters.cuda(), clusters[:, torch.randperm(16384, generator=g)][:, :5000].contiguous().cuda()),
-             ("permuted", a.cuda().permute(0, 2, 1).contiguous().permute(0, 2, 1), b[:, :3000].cuda())]
-    for name, xyz, new in cases:
-        if name == "self":
-            new = xyz
-        for mode in (pcu.DIST_EXPANDED_CUDA, pcu.DIST_DIRECT, pcu.DIST_DIRECT_XYZ):
-            try:
-                _lib.check(_lib.lib.b200pci_debug_set(7, 1))      # k <= 4: two-pass path from small sizes on
-                _lib.check(_lib.lib.b200pci_debug_set(17, 1))
-                i1, d1 = pcu._knn(k, xyz, new, mode, True)
-                _lib.check(_lib.lib.b200pci_debug_set(17, 0))
-                i0, d0 = pcu._knn(k, xyz, new, mode, True)
-            finally:
-                _lib.check(_lib.lib.b200pci_debug_set(17, 0))
-                _lib.check(_lib.lib.b200pci_debug_set(7, 0))
-            assert torch.equal(i1, i0), f"{name} mode {mode}: {int((i1 != i0).sum())} indices differ"
-            assert torch.equal(d1.view(torch.int32), d0.view(torch.int32)), f"{name} mode {mode}"
-        if name == "clusters":   # and against the oracle (form 1 = DIRECT)
-            oi, od = orc.knn_form(1, k, xyz[:1].cpu().numpy(), new[:1].cpu().numpy())
-            np.testing.assert_array_equal(i1[:1].cpu().numpy() if mode == pcu.DIST_DIRECT else
-                                          pcu._knn(k, xyz[:1], new[:1], pcu.DIST_DIRECT, False)[0].cpu().numpy(), oi)
 
 
 def test_knn_exact_mode_equals_estimated(ops):

@@ -51,6 +51,8 @@ def test_abi_argument_errors_without_gpu(lib):
     assert L.b200pci_furthest_point_sampling(0, 10, 4, None, None, None, None) == 0  # empty batch
     assert L.b200pci_group_points(0, 3, 10, 4, 4, None, None, None, None) == 0
     assert L.b200pci_debug_set(99, 0.0) == -1
+    for key in (8, 9, 17):  # keys of removed KNN paths: a stale caller fails instead of running the default
+        assert L.b200pci_debug_set(key, 0.0) == -1 and L.b200pci_debug_set(key, 1.0) == -1
 
 
 def test_new_entry_points_argument_handling_without_gpu(lib):
