@@ -353,7 +353,8 @@ int b200pci_fps_p3d(int B, int P, int M, const float *points, int64_t p_sb, int6
 /* E1-E3: emd_cuda replacements (models/EMD/cuda/emd.cpp:23-27, emd_kernel.cu).                  */
 /* xyz1 [B,n,3], xyz2 [B,m,3] contiguous. match [B,m,n]; temp: scratch of                        */
 /* b200pci_emd_workspace_bytes(B,n,m). Launches on `stream` (the reference uses the legacy       */
-/* default stream, emd_kernel.cu:192).                                                           */
+/* default stream, emd_kernel.cu:192). All four return EINVAL for negative sizes, null pointers   */
+/* or B > 65535 (one grid row per pair).                                                         */
 /* ------------------------------------------------------------------------------------------ */
 size_t b200pci_emd_workspace_bytes(int B, int n, int m);
 int b200pci_emd_approxmatch(int B, int n, int m, const float *xyz1, const float *xyz2,

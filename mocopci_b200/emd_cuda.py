@@ -18,12 +18,21 @@ def _check_pair(xyz1, xyz2):
         raise RuntimeError("xyz1 / xyz2 must be (B, N, 3)")
     if xyz2.size(0) != xyz1.size(0):
         raise RuntimeError("CHECK_EQ failed: xyz2.size(0) == b")
+    if xyz2.device != xyz1.device:
+        raise RuntimeError("xyz1 and xyz2 must be on the same device")
     for t, n in ((xyz1, "xyz1"), (xyz2, "xyz2")):
         if not t.is_contiguous():
             raise RuntimeError(f"{n} must be contiguous")
         if t.dtype != torch.float32:
             raise RuntimeError(f"{n} must be float32")
     return xyz1.size(0), xyz1.size(1), xyz2.size(1)
+
+
+def _check_match(match, b, n, m, xyz1):
+    """The kernels read B*N2*N1 floats of ``match`` in row-major (B, N2, N1) order on xyz1's device."""
+    if (tuple(match.shape) != (b, m, n) or not match.is_contiguous() or match.dtype != torch.float32
+            or match.device != xyz1.device):
+        raise RuntimeError("match must be a contiguous float32 (B, N2, N1) tensor on xyz1's device")
 
 
 def approxmatch_forward(xyz1, xyz2):
@@ -41,8 +50,7 @@ def approxmatch_forward(xyz1, xyz2):
 def matchcost_forward(xyz1, xyz2, match):
     """MatchCostForward, emd_kernel.cu:261-283 -> cost (B)."""
     b, n, m = _check_pair(xyz1, xyz2)
-    if tuple(match.shape) != (b, m, n) or not match.is_contiguous() or match.dtype != torch.float32:
-        raise RuntimeError("match must be a contiguous float32 (B, N2, N1) tensor")
+    _check_match(match, b, n, m, xyz1)
     with _lib.on_device(xyz1):
         cost = torch.empty((b,), dtype=torch.float32, device=xyz1.device)
         ws = _lib.workspace(_L.b200pci_emd_workspace_bytes(b, n, m), xyz1.device)
@@ -68,6 +76,9 @@ def emd_cost(xyz1, xyz2):
 def matchcost_backward(grad_cost, xyz1, xyz2, match):
     """MatchCostBackward, emd_kernel.cu:377-402 -> [grad1 (B,N1,3), grad2 (B,N2,3)]."""
     b, n, m = _check_pair(xyz1, xyz2)
+    _check_match(match, b, n, m, xyz1)
+    if grad_cost.numel() != b or grad_cost.device != xyz1.device:
+        raise RuntimeError("grad_cost must have B elements on xyz1's device")
     grad_cost = grad_cost.contiguous().float()
     with _lib.on_device(xyz1):
         g1 = torch.empty((b, n, 3), dtype=torch.float32, device=xyz1.device)
